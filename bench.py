@@ -292,8 +292,9 @@ def run_reference_cpu(steps, warmup, max_seconds=None):
         "value": PER_GPU_BATCH * len(times) / total, "unit": "images/s", "cores": ref.threads,
         "kind": solver_kind(),
         "sample": f"{len(times)} full steps of the same workload at batch {PER_GPU_BATCH} "
-                  f"(torch CPU conv/autograd on {ref.threads} threads; inverse = reference Cython solver, "
-                  f"batch sharded over {ref.nshards} forked workers)",
+                  f"(torch CPU conv/autograd on {ref.threads} threads; inverse = "
+                  + (f"reference Cython solver, batch sharded over {ref.nshards} forked workers)" if solver_kind() == "reference"
+                     else "oracle C restatement of the reference solver, OpenMP)"),
         "steps": len(times), "ms_per_step": 1e3 * total / len(times),
     }
 
@@ -331,6 +332,24 @@ def main_reference(args):
 # ------------------------------------------------------------------------------------------
 # our arm
 # ------------------------------------------------------------------------------------------
+def dump_outputs(out_dir, runner, slot):
+    """write what the last timed step returned, as float32 .npy files (about 12 MB for the headline workload):
+    per level the latents z and per-sample log-likelihoods of the training batch and the samples of the sampling
+    pass, and the FInC weights after that step's Adam update.  The inputs are seeded, so two builds of the
+    project run with the same arguments can be compared file by file."""
+    import numpy as np
+
+    os.makedirs(out_dir, exist_ok=True)
+    s = runner.slots[slot]
+    arrays = {"weights": runner.stack.flat}
+    for li, lv in enumerate(runner.stack.levels):
+        arrays[f"level{li}_z"] = s.acts[li][lv.n_units]
+        arrays[f"level{li}_logp"] = s.logp[li]
+        arrays[f"level{li}_samples"] = s.sample_out[li]
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().float().cpu().numpy())
+
+
 def algorithmic_bytes(phase, lv, B):
     """SURVEY.md 8(d): fp32, per FastFlowUnit on [B,C,H,W]: forward / backward-input / inverse
     read one tensor and write one (8 B/element); backward-weight reads two (8 B/element,
@@ -639,6 +658,8 @@ def main_ours(args):
         torch.distributed.all_reduce(t, op=torch.distributed.ReduceOp.MAX)
         elapsed_ms = float(t.item())
     value = B * world * K / (elapsed_ms * 1e-3)
+    if args.dump_outputs and rank == 0:   # before the runs below update the weights further
+        dump_outputs(args.dump_outputs, runner, (K - 1) % NSLOT)
 
     # ---- the same K steps with the sampling pass on its own stream (reported next to `value`) ------
     overlap = None
@@ -859,7 +880,13 @@ def main():
     ap.add_argument("--no-overlap", action="store_true", help="skip the overlapped-sampling measurement")
     ap.add_argument("--no-detail", action="store_true", help="skip the per-kernel detail table")
     ap.add_argument("--no-extra", action="store_true", help="skip the other named configurations (extra_workloads)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step to DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of our timed path: it does not apply to --impl reference")
     if args.impl == "reference":
         return main_reference(args)
     return main_ours(args)

@@ -1,7 +1,8 @@
 """Compile the REFERENCE's own CPU inverse solver into oracle/_ref/ (test infrastructure).
 
 Source (read where it lies, never copied into the repo):
-    /root/reference/fastflow/utils/fastflow_inverse/solve_parallel_mc.pyx
+    $FINCFLOW_REFERENCE/fastflow/utils/fastflow_inverse/solve_parallel_mc.pyx
+where FINCFLOW_REFERENCE names a checkout of aditya-v-kallappa/FInCFlow.
 It is the default ``PaddedConv2d.reverse`` of the reference
 (fastflow/layers/conv.py:109-163 -> solve_parallel, .pyx:77-126).  The shipped .so
 files are cp37/cp39; the .pyx compiles unchanged with Cython 3 / numpy 2 / py3.12.
@@ -9,10 +10,10 @@ files are cp37/cp39; the .pyx compiles unchanged with Cython 3 / numpy 2 / py3.1
 As in the reference's setup.py (fastflow/utils/fastflow_inverse/setup.py:1-5) no
 ``-fopenmp`` is passed, so ``prange`` runs on ONE thread -- that is the reference
 as shipped.  Outputs (generated .c, .so) go only to oracle/_ref/, which is
-git-ignored but travels to the GPU box with the gpurun snapshot.
+git-ignored.
 
-/root/reference does not exist on the GPU box: this script is a no-op there and
-the prebuilt file is used.
+Without a reference checkout this script is a no-op and a previously built file, if
+any, is used.
 """
 from __future__ import annotations
 
@@ -23,7 +24,8 @@ import sys
 import sysconfig
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-REF_PYX = "/root/reference/fastflow/utils/fastflow_inverse/solve_parallel_mc.pyx"
+REFERENCE = os.environ.get("FINCFLOW_REFERENCE", "")
+REF_PYX = os.path.join(REFERENCE, "fastflow", "utils", "fastflow_inverse", "solve_parallel_mc.pyx") if REFERENCE else ""
 OUT_DIR = os.path.join(HERE, "_ref")
 MOD = "solve_parallel_mc"
 
@@ -35,7 +37,7 @@ def built_path():
 
 def build(force: bool = False):
     if not os.path.exists(REF_PYX):
-        return built_path()  # GPU box: use what travelled with the snapshot
+        return built_path()  # no reference checkout: use what an earlier build left
     have = built_path()
     if have and not force and os.path.getmtime(have) >= os.path.getmtime(REF_PYX):
         return have

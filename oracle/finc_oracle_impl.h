@@ -7,7 +7,7 @@
  *
  * Every function restates one piece of the reference's algorithm for the FInC
  * hot path in the *stored* weight orientation (no flips), citing the reference
- * file:line it follows (paths relative to /root/reference).
+ * file:line it follows (paths relative to the reference checkout).
  *
  * Layout everywhere: contiguous NCHW.  A tensor is [B, G*C, H, W]; group g owns
  * channels [g*C, (g+1)*C) and has its own weight [C, C, kH, kW] (OIHW) and its

@@ -14,8 +14,9 @@ exactly the library calls the reference performs on CPU tensors:
             used instead (kind "port").
 
 The reference's shipped solver build has no OpenMP (1 thread).  To let the CPU arm use all
-host cores, the batch is sharded over a fork()ed process pool (each worker runs the
-unmodified solver on its shard); `cores` reports the pool size.
+host cores, the batch is then sharded over a fork()ed process pool (each worker runs the
+unmodified solver on its shard).  The C restatement used without that solver is OpenMP-parallel
+itself and runs in the calling process.  `cores` reports the thread count.
 """
 from __future__ import annotations
 
@@ -114,9 +115,11 @@ class ReferenceCpuStack:
         self.z = [torch.randn(batch, lv.channels, lv.height, lv.width, generator=g) for lv in levels]
         self.pool = None
         self.nshards = 1
-        if self.threads > 1:
+        # the reference's solver runs on one thread, so the batch is sharded over forked workers; the C
+        # restatement that stands in for it is OpenMP-parallel already, and forked workers that enter
+        # OpenMP after the parent has used it crawl (20x slower per step on 8 cores) or stall
+        if self.threads > 1 and _get_solver():
             self.nshards = min(self.threads, 32)
-            _get_solver()  # build/load before forking
             self.pool = mp.get_context("fork").Pool(self.nshards)
 
     def close(self):

@@ -1,3 +1,4 @@
+import glob
 import os
 import sys
 
@@ -32,16 +33,20 @@ def pytest_collection_modifyitems(config, items):
 
 
 class Golden:
-    """tests/golden/finc_golden.npz: outputs of the reference's own code
-    (tests/golden/make_golden.py)."""
+    """tests/golden/finc_golden_<part>.npz: outputs of the reference's own code
+    (tests/golden/make_golden.py), whole cases split over files of under 1 MB."""
 
     def __init__(self):
-        self.data = np.load(os.path.join(REPO, "tests", "golden", "finc_golden.npz"))
-        self.names = [str(n) for n in self.data["__index__"]]
+        self.data, self.names = {}, []
+        for path in sorted(glob.glob(os.path.join(REPO, "tests", "golden", "finc_golden_*.npz"))):
+            with np.load(path) as part:
+                self.names += [str(n) for n in part["__index__"]]
+                self.data.update({k: part[k] for k in part.files if k != "__index__"})
+        assert self.names, "tests/golden/finc_golden_*.npz missing"
 
     def case(self, name):
         pre = name + "/"
-        return {k[len(pre):]: self.data[k] for k in self.data.files if k.startswith(pre)}
+        return {k[len(pre):]: v for k, v in self.data.items() if k.startswith(pre)}
 
 
 @pytest.fixture(scope="session")

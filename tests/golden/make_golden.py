@@ -1,12 +1,12 @@
-"""Generate golden fixtures by running the REFERENCE's own Python code (authoring container only).
+"""Generate golden fixtures by running the REFERENCE's own Python code (needs a reference checkout).
 
-    python tests/golden/make_golden.py          # writes tests/golden/finc_golden.npz
+    python tests/golden/make_golden.py          # writes tests/golden/finc_golden_<part>.npz
 
-The reference (/root/reference, read-only, absent on the GPU box) is a set of scripts
+The reference (a checkout of aditya-v-kallappa/FInCFlow named by FINCFLOW_REFERENCE) is a set of scripts
 that import relative to ``fastflow/`` as CWD.  We import its ``layers.conv.PaddedConv2d``
 and ``fastflow.FastFlowUnit`` unmodified through these shims (SURVEY.md section 8c):
 
-  1. ``sys.path.insert(0, /root/reference/fastflow)``
+  1. ``sys.path.insert(0, $FINCFLOW_REFERENCE/fastflow)``
   2. stub ``matplotlib`` (imported by utils/solve_mc.py:3)
   3. ``utils.fastflow_inverse.solve_parallel_mc`` -> the reference's .pyx compiled from
      its own source by oracle/build_ref.py (shipped .so files are cp37/cp39)
@@ -32,13 +32,18 @@ import torch
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 REPO = os.path.dirname(os.path.dirname(HERE))
-REF = "/root/reference/fastflow"
+REFERENCE = os.environ.get("FINCFLOW_REFERENCE", "")
+REF = os.path.join(REFERENCE, "fastflow")
+PART_BYTES = 950_000  # every stored file stays under 1 MB
 sys.path.insert(0, REPO)
 
 
 def import_reference():
     from oracle import build_ref
 
+    if not REFERENCE or not os.path.isdir(REF):
+        sys.exit("set FINCFLOW_REFERENCE to a checkout of aditya-v-kallappa/FInCFlow "
+                 f"(no directory {REF!r})")
     sys.path.insert(0, REF)
     mpl = types.ModuleType("matplotlib")
     mpl.use = lambda *a, **k: None
@@ -178,10 +183,36 @@ def main():
         out[f"{name}/x_from_zs"] = xr.numpy()
         out[f"{name}/orders"] = np.array([code[order]], dtype=np.int32)
 
-    out["__index__"] = np.array(index)
-    path = os.path.join(HERE, "finc_golden.npz")
-    np.savez_compressed(path, **out)
-    print(f"wrote {path}: {len(index)} cases, {os.path.getsize(path) / 1e6:.2f} MB")
+    for path in save_parts(out, index, os.path.join(HERE, "finc_golden")):
+        print(f"wrote {path}: {os.path.getsize(path) / 1e6:.2f} MB")
+
+
+def save_parts(out, index, stem):
+    """np.savez_compressed of whole cases, in order, into stem_0.npz, stem_1.npz, ... of at most PART_BYTES
+    each; every part carries the names of its cases in `__index__`"""
+    import io
+
+    def packed(names):
+        arrays = {k: v for k, v in out.items() if k.split("/")[0] in names}
+        buf = io.BytesIO()
+        np.savez_compressed(buf, __index__=np.array(names), **arrays)
+        return buf.getvalue()
+
+    parts, cur = [], []
+    for name in index:
+        if cur and len(packed(cur + [name])) > PART_BYTES:
+            parts.append(cur)
+            cur = []
+        cur.append(name)
+    parts.append(cur)
+    paths = []
+    for i, names in enumerate(parts):
+        data = packed(names)
+        assert len(data) <= PART_BYTES, (names, len(data))
+        paths.append(f"{stem}_{i}.npz")
+        with open(paths[-1], "wb") as f:
+            f.write(data)
+    return paths
 
 
 if __name__ == "__main__":
