@@ -45,6 +45,7 @@ SYMBOLS = (
     "finc_coupling_apply_f32", "finc_coupling_backward_workspace_bytes", "finc_coupling_backward_f32",
     "finc_inverse_dense_bytes", "finc_inverse_dense_scratch_bytes", "finc_inverse_dense_prepare_f32",
     "finc_inverse_dense_f32", "finc_chain_supported", "finc_chain_f32", "finc_inverse_chain_f32",
+    "finc_inverse_chain_multi_f32",
     "finc_backward_weight_batched_workspace_bytes", "finc_backward_weight_batched_f32",
 )
 
@@ -55,6 +56,13 @@ launch_count = 0  # kernels of ours enqueued through this module (bench.py's gpu
 
 class FincNativeError(RuntimeError):
     pass
+
+
+class FincInverseLevel(ctypes.Structure):
+    """include/fincflow_b200.h: FincInverseLevel (the arguments of finc_inverse_chain_f32)"""
+    _fields_ = [("z", ctypes.c_void_p), ("prepared", ctypes.c_void_p), ("prepared_stride_bytes", ctypes.c_size_t),
+                ("x", ctypes.c_void_p)] + [(n, ctypes.c_int) for n in ("B", "G", "C", "H", "W", "kH", "kW")] + [
+                ("orders", ctypes.c_uint), ("n_units", ctypes.c_int), ("u_first", ctypes.c_int), ("u_step", ctypes.c_int)]
 
 
 def load():
@@ -136,6 +144,8 @@ def load():
                                                      ctypes.c_long, ctypes.c_long, ctypes.c_long, p]
     lib.finc_inverse_chain_f32.restype = i
     lib.finc_inverse_chain_f32.argtypes = [p, p, ctypes.c_size_t, p, i, i, i, i, i, i, i, u, i, i, i, p]
+    lib.finc_inverse_chain_multi_f32.restype = i
+    lib.finc_inverse_chain_multi_f32.argtypes = [ctypes.POINTER(FincInverseLevel), i, p]
     lib.finc_chain_supported.restype = i
     lib.finc_chain_supported.argtypes = [i, i, i, i, i, i, i]
     lib.finc_chain_f32.restype = i
@@ -697,24 +707,52 @@ def backward_weight_batched(dz_units, x_units, out_units, ksize, G=4, orders=ORD
     return out_units
 
 
+def _inverse_level(z, tables, ksize, units, G, orders, out, what):
+    """validated FincInverseLevel for one inverse chain (and its output tensor)"""
+    units = list(units)
+    n = len(units)
+    step = units[1] - units[0] if n > 1 else 1
+    if (n > 1 and step == 0) or any(units[i + 1] - units[i] != step for i in range(n - 1)) or min(units) < 0 \
+            or max(units) >= tables.shape[0]:
+        raise FincNativeError(f"{what}: `units` must be an arithmetic sequence of table rows")
+    B, CT, H, W = (int(v) for v in z.shape)
+    x = torch.empty_like(z) if out is None else out
+    lv = FincInverseLevel(z.data_ptr(), tables.data_ptr(), tables.stride(0) * tables.element_size(), x.data_ptr(),
+                          B, G, CT // G, H, W, int(ksize[0]), int(ksize[1]), orders, n, units[0], step)
+    return lv, x
+
+
 def inverse_chain(z, tables, ksize, units, G=4, orders=ORDERS_UNIT, out=None):
     """x = the inverse of the units `units` (an arithmetic sequence of rows of `tables`, applied in that order) in
     ONE launch; `tables` = [U, nbytes] FINC_PREP_INVERSE tables from prepare_weights.  Raises FincNativeError
     (rc FINC_E_UNSUPPORTED) when the shape is not covered -- callers fall back to one inverse() per unit."""
     z = _prep(z, "z")
     _bind_device(z)
-    units = list(units)
-    n = len(units)
-    step = units[1] - units[0] if n > 1 else 1
-    if (n > 1 and step == 0) or any(units[i + 1] - units[i] != step for i in range(n - 1)) or min(units) < 0 \
-            or max(units) >= tables.shape[0]:
-        raise FincNativeError("inverse_chain: `units` must be an arithmetic sequence of table rows")
-    B, CT, H, W = (int(v) for v in z.shape)
-    x = torch.empty_like(z) if out is None else out
-    _check(load().finc_inverse_chain_f32(z.data_ptr(), tables.data_ptr(), tables.stride(0) * tables.element_size(),
-                                         x.data_ptr(), B, G, CT // G, H, W, int(ksize[0]), int(ksize[1]), orders,
-                                         n, units[0], step, _stream(z)), "finc_inverse_chain_f32")
+    lv, x = _inverse_level(z, tables, ksize, units, G, orders, out, "inverse_chain")
+    _check(load().finc_inverse_chain_f32(lv.z, lv.prepared, lv.prepared_stride_bytes, lv.x, lv.B, lv.G, lv.C, lv.H,
+                                         lv.W, lv.kH, lv.kW, lv.orders, lv.n_units, lv.u_first, lv.u_step, _stream(z)),
+           "finc_inverse_chain_f32")
     return x
+
+
+def inverse_chain_multi(levels, G=4, orders=ORDERS_UNIT):
+    """inverse_chain of several levels in ONE launch: `levels` = [(z, tables, ksize, units, out), ...] on one device
+    and stream (out may be None).  Each result equals inverse_chain(z, tables, ksize, units, out=out) bit for bit.
+    Raises FincNativeError (rc FINC_E_UNSUPPORTED) when the levels are not covered together -- callers fall back to
+    one inverse_chain() per level.  Returns the outputs."""
+    if not levels:
+        raise FincNativeError("inverse_chain_multi: no levels")
+    zs = [_prep(lv[0], "z") for lv in levels]
+    if any(z.device != zs[0].device for z in zs):
+        raise FincNativeError("inverse_chain_multi: all levels must be on one device")
+    _bind_device(zs[0])
+    arr = (FincInverseLevel * len(levels))()
+    outs = []
+    for i, (z, (_, tables, ksize, units, out)) in enumerate(zip(zs, levels)):
+        arr[i], x = _inverse_level(z, tables, ksize, units, G, orders, out, "inverse_chain_multi")
+        outs.append(x)
+    _check(load().finc_inverse_chain_multi_f32(arr, len(levels), _stream(zs[0])), "finc_inverse_chain_multi_f32")
+    return outs
 
 
 def sm_count() -> int:

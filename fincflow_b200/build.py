@@ -20,7 +20,7 @@ OUT_DIR = os.path.join(HERE, "lib")
 LIB = os.path.join(OUT_DIR, "libfincflow_b200.so")
 SOURCES = [f"finc_inverse_rw_c{c}k{k}.cu" for c, k in ((12, 5), (12, 3), (6, 5), (6, 3), (4, 5), (3, 5), (4, 3),
                                                       (3, 3), (2, 5), (2, 3), (1, 5), (1, 3))] + [  # heaviest first
-    "finc_api.cu", "finc_naive.cu", "finc_conv.cu", "finc_inverse.cu", "finc_inverse_wave.cu", "finc_inverse_rw.cu",
+    "finc_inverse_rw_multi.cu", "finc_api.cu", "finc_naive.cu", "finc_conv.cu", "finc_inverse.cu", "finc_inverse_wave.cu", "finc_inverse_rw.cu",
     "finc_wgrad.cu", "finc_collective.cu", "finc_affine.cu", "finc_chain.cu", "tc_api.cu", "tc_wgrad.cu",
     *[f"tc_igemm_nhwc_p{p}_c{c}.cu" for p in (3, 1) for c in (1, 2, 4)], "tc_igemm_rows_p3.cu", "tc_igemm_rows_p1.cu"] + [
     f"finc_inverse_wave_c{c}.cu" for c in (24, 12, 6, 4, 3, 2, 1)] + [  # heaviest first

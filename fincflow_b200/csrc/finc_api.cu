@@ -217,6 +217,22 @@ int finc_inverse_chain_f32(const float* z, const void* prepared, size_t prepared
     return handled ? FINC_OK : FINC_E_UNSUPPORTED;
 }
 
+int finc_inverse_chain_multi_f32(const FincInverseLevel* levels, int n_levels, void* stream) {
+    if (!levels || n_levels < 1) return FINC_E_BADARG;
+    if (n_levels > kInverseMultiMaxLevels) return FINC_E_UNSUPPORTED;
+    RwChainLevel lv[kInverseMultiMaxLevels];
+    for (int i = 0; i < n_levels; ++i) {
+        const FincInverseLevel& l = levels[i];
+        if (!shape_ok(l.B, l.G, l.C, l.H, l.W, l.kH, l.kW) || !l.prepared || l.n_units < 1 ||
+            l.prepared_stride_bytes % 16 != 0)
+            return FINC_E_BADARG;
+        if (l.B > 0 && (!l.z || !l.x)) return FINC_E_BADARG;
+        lv[i] = RwChainLevel{l.z, (const float*)l.prepared, l.x, mk(l.B, l.G, l.C, l.H, l.W, l.kH, l.kW, l.orders),
+                             l.n_units, l.u_first, l.u_step, (long)(l.prepared_stride_bytes / 4)};
+    }
+    return launch_inverse_rw_multi(lv, n_levels, (cudaStream_t)stream);
+}
+
 int finc_apply_grad_mask_f32(float* dw, int G, int C, int kH, int kW, unsigned orders, void* stream) {
     if (!shape_ok(1, G, C, 1, 1, kH, kW) || !dw) return FINC_E_BADARG;
     return launch_mask(dw, mk(1, G, C, 1, 1, kH, kW, orders), (cudaStream_t)stream);

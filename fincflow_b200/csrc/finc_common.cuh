@@ -186,6 +186,17 @@ int launch_inverse_rw(const float* z, const float* w, float* x, const Shape& s, 
                       bool* handled);
 int launch_inverse_rw_chain(const float* z, const float* w, float* x, const Shape& s, bool prepared, int n_units,
                             int u_first, int u_step, long unit_stride, cudaStream_t st, bool* handled);
+// one level of launch_inverse_rw_multi: the arguments of launch_inverse_rw_chain (prepared tables)
+struct RwChainLevel {
+    const float* z;
+    const float* w;
+    float* x;
+    Shape s;
+    int n_units, u_first, u_step;
+    long unit_stride;
+};
+constexpr int kInverseMultiMaxLevels = 4;
+int launch_inverse_rw_multi(const RwChainLevel* levels, int n, cudaStream_t st);
 bool rw_shape_supported(const Shape& s);
 size_t wave_prepared_floats(const Shape& s);
 int launch_wave_prepare(const float* w, float* out, int n_units, size_t w_stride, size_t out_stride, const Shape& s,

@@ -50,10 +50,19 @@ int launch_inverse_rw(const float* z, const float* w, float* x, const Shape& s, 
     return launch_inverse_rw_chain(z, w, x, s, prepared, 1, 0, 1, 0, st, handled);
 }
 
-// n_units > 1: a chain of units solved in place in one launch (prepared tables, unit u at w + u * unit_stride)
-int launch_inverse_rw_chain(const float* z, const float* w, float* x, const Shape& s, bool prepared, int n_units,
-                            int u_first, int u_step, long unit_stride, cudaStream_t st, bool* handled) {
-    *handled = false;
+namespace {
+// what the per-level planner picks for one launch of the kernel
+struct RwPlan {
+    RwArgs a;
+    int P, nwarps;
+    dim3 grid;
+    size_t smem, wk_bytes, stage_bytes;
+};
+
+// plans one level's launch; *planned = false (rc 0) when the register-window kernel does not cover it
+int plan_inverse_rw(const float* z, const float* w, float* x, const Shape& s, bool prepared, int n_units, int u_first,
+                    int u_step, long unit_stride, RwPlan& plan, bool* planned) {
+    *planned = false;
     if (n_units > 1 && !prepared) return FINC_E_UNSUPPORTED;
     static const int enabled = env_int("FINC_RW", 1);
     if (!enabled) return 0;
@@ -151,8 +160,30 @@ int launch_inverse_rw_chain(const float* z, const float* w, float* x, const Shap
     a.S = env_int("FINC_RW_S", a.S);
     const size_t smem = wk_bytes + (size_t)nwarps * a.S * (stage_bytes + 8) + 8 + 16;
     if (smem > budget + 2048) return prepared ? FINC_E_UNSUPPORTED : 0;
-    dim3 grid((unsigned)ctas, a.gsplit ? s.G : 1, 1);
-    int rc;
+    plan.a = a;
+    plan.P = P;
+    plan.nwarps = nwarps;
+    plan.grid = dim3((unsigned)ctas, a.gsplit ? s.G : 1, 1);
+    plan.smem = smem;
+    plan.wk_bytes = wk_bytes;
+    plan.stage_bytes = stage_bytes;
+    *planned = true;
+    return 0;
+}
+}  // namespace
+
+// n_units > 1: a chain of units solved in place in one launch (prepared tables, unit u at w + u * unit_stride)
+int launch_inverse_rw_chain(const float* z, const float* w, float* x, const Shape& s, bool prepared, int n_units,
+                            int u_first, int u_step, long unit_stride, cudaStream_t st, bool* handled) {
+    *handled = false;
+    RwPlan plan;
+    bool planned = false;
+    int rc = plan_inverse_rw(z, w, x, s, prepared, n_units, u_first, u_step, unit_stride, plan, &planned);
+    if (rc || !planned) return rc;
+    const RwArgs& a = plan.a;
+    const int C = s.C, KS = s.kH, P = plan.P, nwarps = plan.nwarps;
+    const dim3 grid = plan.grid;
+    const size_t smem = plan.smem;
     if (KS == 3) {
         switch (C) {
             case 1: rc = rw::dispatch_ck<1, 3>(P, a, grid, nwarps, smem, st); break;
@@ -175,6 +206,49 @@ int launch_inverse_rw_chain(const float* z, const float* w, float* x, const Shap
     if (rc == FINC_E_UNSUPPORTED) return prepared ? FINC_E_UNSUPPORTED : 0;
     *handled = true;
     return rc;
+}
+
+// The sampling chains of several levels in ONE launch of inverse_rw_multi_kernel.  Every level keeps the P, NSTK and T
+// its own launch would use (so every tile sees the same arithmetic, bit for bit); its CTAs of 6 warps are sized so
+// that each warp solves at most one item, and the launch is refused unless all CTAs are resident at once.
+int launch_inverse_rw_multi(const RwChainLevel* lv, int n, cudaStream_t st) {
+    if (n < 1 || n > rw::kRwMultiLevels) return FINC_E_UNSUPPORTED;
+    rw::RwMultiArgs m{};
+    constexpr int NW = rw::kRwMultiWarps;
+    size_t smem = 0;
+    int ctas = 0, nl = 0;
+    for (int i = 0; i < n; ++i) {
+        const RwChainLevel& c = lv[i];
+        if (c.s.B == 0) continue;
+        RwPlan plan;
+        bool planned = false;
+        const int rc = plan_inverse_rw(c.z, c.w, c.x, c.s, true, c.n_units, c.u_first, c.u_step, c.unit_stride, plan,
+                                       &planned);
+        if (rc || !planned) return FINC_E_UNSUPPORTED;
+        const int C = c.s.C, KS = c.s.kH, P = plan.P;
+        int kind = -1;
+        if (C == rw::RwKind0::C && KS == rw::RwKind0::KS && P == rw::RwKind0::P) kind = 0;
+        if (C == rw::RwKind1::C && KS == rw::RwKind1::KS && P == rw::RwKind1::P) kind = 1;
+        if (C == rw::RwKind2::C && KS == rw::RwKind2::KS && P == rw::RwKind2::P) kind = 2;
+        if (kind < 0 || plan.a.T != 1) return FINC_E_UNSUPPORTED;   // (multi-tile stacks: not instantiated)
+        RwArgs a = plan.a;
+        a.S = 1;
+        const long vgrid = (a.n_items + NW - 1) / NW;
+        const long lctas = vgrid * plan.grid.y;
+        m.lv[nl] = a;
+        m.kind[nl] = kind;
+        m.vgrid[nl] = (int)vgrid;
+        m.first[nl] = ctas;
+        ctas += (int)lctas;
+        const size_t need = plan.wk_bytes + (size_t)NW * (plan.stage_bytes + 8) + 8 + 16;
+        if (need > smem) smem = need;
+        ++nl;
+    }
+    if (nl == 0) return 0;
+    for (int i = nl; i <= rw::kRwMultiLevels; ++i) m.first[i] = ctas;
+    if (smem > max_optin_smem_cached()) return FINC_E_UNSUPPORTED;
+    if (ctas > (long)rw::multi_ctas_per_sm(smem) * sm_count_cached()) return FINC_E_UNSUPPORTED;
+    return rw::launch_multi(m, ctas, smem, st);
 }
 
 }  // namespace finc

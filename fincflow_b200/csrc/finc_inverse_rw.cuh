@@ -71,15 +71,18 @@ struct Cfg {
     static constexpr int MAXW = EST <= 100 ? 16 : 8;   // (12 warps with shallower stacks measured slower)
 };
 
+// The whole solve of one launch's share of a level.  (vblock, vgrid) take the place of (blockIdx.x, gridDim.x) and
+// grp that of blockIdx.y (the group of a gsplit launch), so that one launch can host several levels.
 // MT: stacks hold more than one tile (large batches).  With one tile per stack the window never
 // has to be cleared at a tile top and the row pointer never wraps, which shortens the step.
-template <int C, int KH, int KW, int P, bool MT>
-__global__ void __launch_bounds__(Cfg<C, KH, KW, P>::MAXW * 32, 1) inverse_rw_kernel(const RwArgs a) {
+// WREG / CREG: tap / corner weights held in registers (sign folded in) instead of read from the shared-memory table;
+// x * (-w) and (-x) * w round identically, so both give the same bits.
+template <int C, int KH, int KW, int P, bool MT, bool WREG, bool CREG>
+__device__ __forceinline__ void inverse_rw_body(const RwArgs& a, int vblock, int vgrid, int grp) {
     using K = Cfg<C, KH, KW, P>;
     constexpr int CL = K::CL;
     constexpr int CPP = Pad4<C>::value;
     constexpr int TS = Pad4<C>::tap_stride;
-    constexpr bool WREG = K::WREG, CREG = K::CREG;
 
     extern __shared__ __align__(128) unsigned char smem_raw[];
     float* wk = reinterpret_cast<float*>(smem_raw);
@@ -98,9 +101,9 @@ __global__ void __launch_bounds__(Cfg<C, KH, KW, P>::MAXW * 32, 1) inverse_rw_ke
     uint64_t* bars = bar0 + warp * a.S;
     uint64_t* wbar = bar0 + nwarps * a.S;
 
-    const int g_fixed = a.gsplit ? (int)blockIdx.y : -1;
-    const long gw = (long)warp * gridDim.x + blockIdx.x;
-    const long gstride = (long)gridDim.x * nwarps;
+    const int g_fixed = a.gsplit ? grp : -1;
+    const long gw = (long)warp * vgrid + vblock;
+    const long gstride = (long)vgrid * nwarps;
 
     auto item_g = [&](long item) -> int { return a.gsplit ? g_fixed : (int)(item % s.G); };
     auto item_n0 = [&](long item) -> int { return (int)(a.gsplit ? item : item / s.G) * item_tiles; };
@@ -126,7 +129,7 @@ __global__ void __launch_bounds__(Cfg<C, KH, KW, P>::MAXW * 32, 1) inverse_rw_ke
     pdl_wait();
     pdl_trigger();
     if (a.prepared && threadIdx.x == 0) {  // the whole weight table of every unit of the chain: one bulk copy each
-        if (blockIdx.x == 0 && blockIdx.y == 0) {   // refuse a table of another kind / layout
+        if (vblock == 0 && grp == 0) {   // refuse a table of another kind / layout
             const float* h = a.w + (long)a.u_first * a.unit_stride;
             if (__ldg(h) != 1179208259.f || (int)__ldg(h + 1) != 2 || (int)__ldg(h + 2) != CPP || (int)__ldg(h + 3) != TS) __trap();
         }
@@ -395,6 +398,62 @@ __global__ void __launch_bounds__(Cfg<C, KH, KW, P>::MAXW * 32, 1) inverse_rw_ke
     if (a.bulk) bulk_wait_all();
     if (threadIdx.x == 0) dbg_mark(a.dbg, 4);
 }
+
+template <int C, int KH, int KW, int P, bool MT>
+__global__ void __launch_bounds__(Cfg<C, KH, KW, P>::MAXW * 32, 1) inverse_rw_kernel(const RwArgs a) {
+    using K = Cfg<C, KH, KW, P>;
+    inverse_rw_body<C, KH, KW, P, MT, K::WREG, K::CREG>(a, (int)blockIdx.x, (int)gridDim.x, (int)blockIdx.y);
+}
+
+// ---- several levels in one launch (finc_inverse_chain_multi_f32) ------------------------------------------------
+// Every level of a stack has independent inputs, and one level's chain leaves most of the GPU idle at small batches
+// (a dependent 16-unit x (H+W-1)-step chain per warp, few warps per SM).  One launch hosts the warp items of all
+// levels at once: CTA b belongs to the level l with first[l] <= b < first[l+1] and runs the body of its kind.  The
+// cap of 2 CTAs x 6 warps per SM (<= 168 registers) is why the C = 6 taps and the C = 12 corner come from the
+// shared-memory table here.
+constexpr int kRwMultiLevels = kInverseMultiMaxLevels;
+constexpr int kRwMultiWarps = 6;    // warps per CTA
+
+struct RwMultiArgs {
+    RwArgs lv[kRwMultiLevels];
+    int first[kRwMultiLevels + 1];  // CTAs of level l: [first[l], first[l+1]); first[n] = grid size
+    int vgrid[kRwMultiLevels];      // CTAs per group slice of level l
+    int kind[kRwMultiLevels];       // which body (template argument) solves level l
+};
+
+// one (C, K, P) body of the multi-level kernel
+template <int C_, int K_, int P_, bool WREG_, bool CREG_>
+struct RwKind {
+    static constexpr int C = C_, KS = K_, P = P_;
+    static constexpr bool WREG = WREG_, CREG = CREG_;
+};
+
+template <class K>
+__device__ __forceinline__ void run_kind(const RwArgs& a, int vblock, int vgrid, int grp) {
+    inverse_rw_body<K::C, K::KS, K::KS, K::P, false, K::WREG, K::CREG>(a, vblock, vgrid, grp);
+}
+
+template <class K0, class K1, class K2>
+__global__ void __launch_bounds__(kRwMultiWarps * 32, 2) inverse_rw_multi_kernel(const RwMultiArgs m) {
+    const int b = (int)blockIdx.x;
+    int l = 0;
+#pragma unroll
+    for (int i = 1; i < kRwMultiLevels; ++i) l += b >= m.first[i];
+    const int r = b - m.first[l], vg = m.vgrid[l];
+    switch (m.kind[l]) {
+        case 0: run_kind<K0>(m.lv[l], r % vg, vg, r / vg); break;
+        case 1: run_kind<K1>(m.lv[l], r % vg, vg, r / vg); break;
+        default: run_kind<K2>(m.lv[l], r % vg, vg, r / vg); break;
+    }
+}
+
+// the kinds instantiated: the levels of cifar10_levels / imagenet32_levels at k = 3 ([12,16,16], [24,8,8], [48,4,4];
+// C = 3, 6, 12 per group) with the P the per-level planner picks for them
+using RwKind0 = RwKind<3, 3, 1, true, true>;
+using RwKind1 = RwKind<6, 3, 2, false, true>;
+using RwKind2 = RwKind<12, 3, 4, false, false>;
+int launch_multi(const RwMultiArgs& m, int n_ctas, size_t smem, cudaStream_t st);   // finc_inverse_rw_multi.cu
+int multi_ctas_per_sm(size_t smem);   // CTAs of the multi-level kernel one SM holds with `smem` bytes each (0 on error)
 
 template <int C, int KH, int KW, int P>
 int launch_inst(const RwArgs& a, dim3 grid, int nwarps, size_t smem, cudaStream_t st) {

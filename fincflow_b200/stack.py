@@ -193,7 +193,7 @@ class HotPathRunner:
     def __init__(self, stack: FincStack, batch: int, device, slots=1, lr=1e-3, host_io=False,
                  process_group=None, use_graphs=True, use_prepared=True, fused_collective=True,
                  device_latents=False, overlap_sampling=False, dense_inverse=False, level_parallel=False, chain=True,
-                 batched_wgrad=True):
+                 batched_wgrad=True, multi_level_inverse=True):
         self.stack, self.B, self.device = stack, batch, torch.device(device)
         # chain: the forward pass of a level and its backward-data chain are ONE launch each (finc_chain_f32: the
         # image tiles stay in shared memory between units; all activations are still written) wherever the shape
@@ -208,6 +208,11 @@ class HotPathRunner:
             self.wg_batched.append(torch.zeros(nb, dtype=torch.uint8, device=self.device) if nb else None)
         self.inv_chain = [0] * len(stack.levels)   # units per inverse-chain launch: _probe_inverse_chain(), once the tables exist
         self._want_inv_chain = chain
+        # multi_level_inverse: when every level's sampling chain is one whole launch, the chains of all levels run in
+        # ONE launch (finc_inverse_chain_multi_f32; bit-identical): at small batches one level's chain leaves most
+        # SMs idle, so the levels run side by side instead of one after another.  Set by _probe_inverse_chain().
+        self._want_inv_multi = multi_level_inverse
+        self.inv_multi = False
         # level_parallel: the levels of a FincStack have independent inputs, so their unit chains (forward,
         # dX, inverse) may run next to each other -- one stream per level, forked from and joined to the
         # current stream (inside a graph: parallel branches).  Batch-256 launches are latency-bound and do not
@@ -491,7 +496,21 @@ class HotPathRunner:
         self._prepare_weights()
 
     def _inverse(self, s):
+        if self.inv_multi:
+            if self.device_latents:
+                for z in s.zin:
+                    z.normal_()
+            self._inverse_multi(s)
+            return
         self._per_level(lambda li, lv: self._inverse_level(s, li, lv))
+
+    def _inverse_multi(self, s):
+        """the whole sampling chain of every level in one launch, into the buffer the per-level path ends in"""
+        outs = _native.inverse_chain_multi([
+            (s.zin[li], self.tables[li][_native.PREP_INVERSE], lv.kernel_size, range(lv.n_units - 1, -1, -1),
+             s.samp[li][(lv.n_units - 1) % 2]) for li, lv in enumerate(self.stack.levels)])
+        for li, x in enumerate(outs):
+            s.sample_out[li] = x
 
     def _inverse_level(self, s, li, lv):
         if self.device_latents:
@@ -563,6 +582,14 @@ class HotPathRunner:
                     break
                 except _native.FincNativeError:
                     pass
+        self.inv_multi = False
+        if self._want_inv_multi and len(self.stack.levels) > 1 and not self.dense and \
+                all(m == lv.n_units for m, lv in zip(self.inv_chain, self.stack.levels)):
+            try:
+                self._inverse_multi(s)
+                self.inv_multi = True
+            except _native.FincNativeError:
+                pass
 
     def _prepare_warm_and_capture(self):
         self._prepare_weights()

@@ -330,6 +330,24 @@ int finc_inverse_chain_f32(const float* z, const void* prepared, size_t prepared
                            int C, int H, int W, int kH, int kW, unsigned orders, int n_units, int u_first, int u_step,
                            void* stream);
 
+/* The sampling chains of several levels (independent inputs, e.g. the levels of a multi-scale flow) in ONE launch:
+ * level i is what finc_inverse_chain_f32 with levels[i]'s arguments computes, bit for bit.  The warp items of all
+ * levels run side by side, so small batches -- where one level's chain leaves most SMs idle -- take about as long as
+ * the slowest level instead of the sum.  Levels with B = 0 are skipped.  FINC_E_UNSUPPORTED when a level is not one
+ * of the instantiated kinds (kH = kW = 3 and (C, P) = (3, 1), (6, 2), (12, 4), P being what the single-level launch
+ * picks), when n_levels > 4, or when the levels do not fit on the GPU at once (shared memory per CTA,
+ * every CTA resident); call finc_inverse_chain_f32 per level then. */
+typedef struct FincInverseLevel {
+    const float* z;
+    const void* prepared;
+    size_t prepared_stride_bytes;
+    float* x;
+    int B, G, C, H, W, kH, kW;
+    unsigned orders;
+    int n_units, u_first, u_step;
+} FincInverseLevel;
+int finc_inverse_chain_multi_f32(const FincInverseLevel* levels, int n_levels, void* stream);
+
 int finc_chain_supported(int G, int C, int H, int W, int kH, int kW, int with_affine);
 int finc_chain_f32(const float* x, const float* w, long w_stride, float* y, long y_stride, const float* A,
                    const float* bias, float* logdet, int B, int G, int C, int H, int W, int kH, int kW,
