@@ -6,6 +6,7 @@ Public surface (mirrors the reference's fastflow package for this path):
     FlowSequential                                               fastflow/layers/flowsequential.py
     PaddedConv2d                                                 fastflow/layers/conv.py
     FastFlowUnit, clear_grad                                     fastflow/fastflow.py, train/experiment.py:16-18
+    weight_grad_in_reverse                                       (reverse records a graph for the weights alone)
     flows.FastFlow (+ fastflow_mnist / _cifar10 / _imagenet32 / _imagenet64 builders)
 
 Everything computes through the C ABI in include/fincflow_b200.h (libfincflow_b200.so, hand-written
@@ -22,6 +23,7 @@ _LAZY = {
     "PaddedConv2d": ("layers.conv", "PaddedConv2d"),
     "FastFlowUnit": ("fastflow", "FastFlowUnit"),
     "clear_grad": ("fastflow", "clear_grad"),
+    "weight_grad_in_reverse": ("ops", "weight_grad_in_reverse"),
     "FastFlow": ("flows", "FastFlow"),
     "GaussianPrior": ("flows", "GaussianPrior"),
     "fastflow_mnist": ("flows", "fastflow_mnist"),

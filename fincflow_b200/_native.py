@@ -30,13 +30,14 @@ FLAG_QUARTER_GPU = 128
 FLAG_HALF_GPU = 256
 FLAG_WAVE_SMEM = 512
 FLAG_TF32_1PASS = 1024
+FLAG_NEGATE = 4096
 PREP_FORWARD, PREP_BACKWARD_INPUT, PREP_INVERSE = 0, 1, 2
 
 # every symbol declared in include/fincflow_b200.h
 SYMBOLS = (
     "finc_abi_version", "finc_error_string", "finc_set_device", "finc_sm_count",
     "finc_forward_f32", "finc_backward_input_f32", "finc_backward_weight_workspace_bytes",
-    "finc_backward_weight_f32", "finc_inverse_f32", "finc_apply_grad_mask_f32", "finc_logdet_f32",
+    "finc_backward_weight_f32", "finc_inverse_f32", "finc_inverse_adjoint_f32", "finc_apply_grad_mask_f32", "finc_logdet_f32",
     "finc_gaussian_logp_f32", "finc_debug_timestamps", "finc_prepared_weights_bytes", "finc_prepare_weights_f32",
     "finc_squeeze_f32", "finc_unsqueeze_f32", "finc_adam_step_f32", "finc_allreduce_adam_f32", "finc_affine1x1_f32",
     "finc_affine1x1_backward_weight_workspace_bytes", "finc_affine1x1_backward_weight_f32",
@@ -88,6 +89,7 @@ def load():
     lib.finc_backward_weight_workspace_bytes.argtypes = dims
     lib.finc_backward_weight_f32.argtypes = [p, p, p, p, sz, *dims, u, u, p]
     lib.finc_inverse_f32.argtypes = [p, p, p, *dims, u, u, p]
+    lib.finc_inverse_adjoint_f32.argtypes = [p, p, p, *dims, u, u, p]
     lib.finc_apply_grad_mask_f32.argtypes = [p, i, i, i, i, u, p]
     lib.finc_logdet_f32.argtypes = [p, p, *dims, u, p]
     lib.finc_gaussian_logp_f32.argtypes = [p, p, p, p, ctypes.c_float, i, ctypes.c_long, p]
@@ -157,7 +159,7 @@ def load():
     lib.finc_coupling_apply_f32.restype = i
     lib.finc_coupling_apply_f32.argtypes = [p, p, p, p, p, sz, i, i, i, i, i, i, u, p]
     for f in ("finc_set_device", "finc_forward_f32", "finc_backward_input_f32", "finc_backward_weight_f32",
-              "finc_inverse_f32", "finc_apply_grad_mask_f32", "finc_logdet_f32", "finc_gaussian_logp_f32"):
+              "finc_inverse_f32", "finc_inverse_adjoint_f32", "finc_apply_grad_mask_f32", "finc_logdet_f32", "finc_gaussian_logp_f32"):
         getattr(lib, f).restype = i
     if lib.finc_abi_version() != 1:
         raise FincNativeError("libfincflow_b200.so ABI version mismatch; rebuild")
@@ -300,6 +302,19 @@ def inverse(z, w, G=4, orders=ORDERS_UNIT, flags=0, out=None, prepared=None, ksi
     _check(load().finc_inverse_f32(z.data_ptr(), w.data_ptr(), x.data_ptr(), *d, orders, flags, _stream(z)),
            "finc_inverse_f32")
     return x
+
+
+def inverse_adjoint(dx, w, G=4, orders=ORDERS_UNIT, flags=0, out=None):
+    """dz = A^-T dx, the adjoint of inverse() (x = A^-1 z): <dx, inverse(z)> == <inverse_adjoint(dx), z>.
+    `out` may be `dx` (in place).  C ABI: finc_inverse_adjoint_f32."""
+    dx = _prep(dx, "dx")
+    w = _prep(w, "weight")
+    d = _dims(dx, w, G)
+    _bind_device(dx)
+    dz = torch.empty_like(dx) if out is None else out
+    _check(load().finc_inverse_adjoint_f32(dx.data_ptr(), w.data_ptr(), dz.data_ptr(), *d, orders, flags, _stream(dx)),
+           "finc_inverse_adjoint_f32")
+    return dz
 
 
 def apply_grad_mask_(dw, G, orders):

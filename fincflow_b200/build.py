@@ -18,8 +18,9 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OUT_DIR = os.path.join(HERE, "lib")
 LIB = os.path.join(OUT_DIR, "libfincflow_b200.so")
-SOURCES = [f"finc_inverse_rw_c{c}k{k}.cu" for c, k in ((12, 5), (12, 3), (6, 5), (6, 3), (4, 5), (3, 5), (4, 3),
-                                                      (3, 3), (2, 5), (2, 3), (1, 5), (1, 3))] + [  # heaviest first
+SOURCES = [f"finc_inverse_rw_{adj}c{c}k{k}.cu" for c, k in ((12, 5), (12, 3), (6, 5), (6, 3), (4, 5), (3, 5), (4, 3),
+                                                            (3, 3), (2, 5), (2, 3), (1, 5), (1, 3))
+           for adj in ("", "adj_")] + [  # heaviest first; each inverse family with its adjoint
     "finc_inverse_rw_multi.cu", "finc_api.cu", "finc_naive.cu", "finc_conv.cu", "finc_inverse.cu", "finc_inverse_wave.cu", "finc_inverse_rw.cu",
     "finc_wgrad.cu", "finc_collective.cu", "finc_affine.cu", "finc_chain.cu", "tc_api.cu", "tc_wgrad.cu",
     *[f"tc_igemm_nhwc_p{p}_c{c}.cu" for p in (3, 1) for c in (1, 2, 4)], "tc_igemm_rows_p3.cu", "tc_igemm_rows_p1.cu"] + [

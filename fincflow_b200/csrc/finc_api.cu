@@ -203,6 +203,24 @@ int finc_inverse_f32(const float* z, const float* w, float* x, int B, int G, int
     return rc;
 }
 
+int finc_inverse_adjoint_f32(const float* dx, const float* w, float* dz, int B, int G, int C, int H, int W, int kH,
+                             int kW, unsigned orders, unsigned flags, void* stream) {
+    if (!shape_ok(B, G, C, H, W, kH, kW) || !w) return FINC_E_BADARG;
+    if (flags & FINC_FLAG_PREPARED) return FINC_E_UNSUPPORTED;
+    if (B == 0) return FINC_OK;
+    if (!dx || !dz) return FINC_E_BADARG;
+    // A^T is the inverse swept from the opposite corner: flip both order bits of every group
+    const unsigned flip = G >= 16 ? 0xFFFFFFFFu : (1u << (2 * G)) - 1u;
+    const Shape s = mk(B, G, C, H, W, kH, kW, orders ^ flip);
+    cudaStream_t st = (cudaStream_t)stream;
+    int rc = 0;
+    bool handled = false;
+    if (!(flags & FINC_FLAG_NAIVE)) rc = launch_inverse_rw_adjoint(dx, w, dz, s, st, &handled);
+    if (rc) return rc;
+    if (!handled) rc = launch_inverse_adjoint_naive(dx, w, dz, s, st);
+    return rc;
+}
+
 int finc_inverse_chain_f32(const float* z, const void* prepared, size_t prepared_stride_bytes, float* x, int B, int G,
                            int C, int H, int W, int kH, int kW, unsigned orders, int n_units, int u_first, int u_step,
                            void* stream) {

@@ -184,6 +184,8 @@ int launch_inverse_wave(const float* z, const float* w, float* x, const Shape& s
                         bool* handled);
 int launch_inverse_rw(const float* z, const float* w, float* x, const Shape& s, bool prepared, cudaStream_t st,
                       bool* handled);
+int launch_inverse_rw_adjoint(const float* dx, const float* w, float* dz, const Shape& s, cudaStream_t st,
+                              bool* handled);
 int launch_inverse_rw_chain(const float* z, const float* w, float* x, const Shape& s, bool prepared, int n_units,
                             int u_first, int u_step, long unit_stride, cudaStream_t st, bool* handled);
 // one level of launch_inverse_rw_multi: the arguments of launch_inverse_rw_chain (prepared tables)
@@ -212,6 +214,7 @@ int launch_wgrad_batched(const float* dz, const float* x, float* dw, float* work
 
 int launch_conv_naive(const float* x, const float* w, float* y, const Shape& s, bool transpose, cudaStream_t st);
 int launch_inverse_naive(const float* z, const float* w, float* x, const Shape& s, cudaStream_t st);
+int launch_inverse_adjoint_naive(const float* dx, const float* w, float* dz, const Shape& s, cudaStream_t st);
 int launch_wgrad_naive(const float* dz, const float* x, float* dw, const Shape& s, unsigned flags, cudaStream_t st);
 int launch_mask(float* dw, const Shape& s, cudaStream_t st);
 int launch_logdet(const float* w, float* logdet, bool accumulate, const Shape& s, cudaStream_t st);

@@ -1,5 +1,5 @@
 // finc_inverse_rw.cu -- host-side planning for the register-window wavefront inverse
-// (kernel: finc_inverse_rw.cuh; instantiations: finc_inverse_rw_c<N>k<K>.cu).
+// (kernel: finc_inverse_rw.cuh; instantiations: finc_inverse_rw_c<N>k<K>.cu, adjoint: finc_inverse_rw_adj_c<N>k<K>.cu).
 #include "finc_inverse_rw.cuh"
 
 #include <cstdlib>
@@ -9,7 +9,9 @@ namespace finc {
 namespace rw {
 #define FINC_RW_EXTERN(C)                                                                                   \
     extern template int dispatch_ck<C, 3>(int, const RwArgs&, dim3, int, size_t, cudaStream_t);             \
-    extern template int dispatch_ck<C, 5>(int, const RwArgs&, dim3, int, size_t, cudaStream_t);
+    extern template int dispatch_ck<C, 5>(int, const RwArgs&, dim3, int, size_t, cudaStream_t);             \
+    extern template int dispatch_ck<C, 3, true>(int, const RwArgs&, dim3, int, size_t, cudaStream_t);       \
+    extern template int dispatch_ck<C, 5, true>(int, const RwArgs&, dim3, int, size_t, cudaStream_t);
 FINC_RW_EXTERN(1)
 FINC_RW_EXTERN(2)
 FINC_RW_EXTERN(3)
@@ -170,6 +172,33 @@ int plan_inverse_rw(const float* z, const float* w, float* x, const Shape& s, bo
     *planned = true;
     return 0;
 }
+
+// the instantiation of the planned (C, K) family
+template <bool ADJ>
+int dispatch_plan(const RwPlan& plan, const Shape& s, cudaStream_t st) {
+    const RwArgs& a = plan.a;
+    const int P = plan.P, nwarps = plan.nwarps;
+    const dim3 grid = plan.grid;
+    const size_t smem = plan.smem;
+    if (s.kH == 3) {
+        switch (s.C) {
+            case 1: return rw::dispatch_ck<1, 3, ADJ>(P, a, grid, nwarps, smem, st);
+            case 2: return rw::dispatch_ck<2, 3, ADJ>(P, a, grid, nwarps, smem, st);
+            case 3: return rw::dispatch_ck<3, 3, ADJ>(P, a, grid, nwarps, smem, st);
+            case 4: return rw::dispatch_ck<4, 3, ADJ>(P, a, grid, nwarps, smem, st);
+            case 6: return rw::dispatch_ck<6, 3, ADJ>(P, a, grid, nwarps, smem, st);
+            default: return rw::dispatch_ck<12, 3, ADJ>(P, a, grid, nwarps, smem, st);
+        }
+    }
+    switch (s.C) {
+        case 1: return rw::dispatch_ck<1, 5, ADJ>(P, a, grid, nwarps, smem, st);
+        case 2: return rw::dispatch_ck<2, 5, ADJ>(P, a, grid, nwarps, smem, st);
+        case 3: return rw::dispatch_ck<3, 5, ADJ>(P, a, grid, nwarps, smem, st);
+        case 4: return rw::dispatch_ck<4, 5, ADJ>(P, a, grid, nwarps, smem, st);
+        case 6: return rw::dispatch_ck<6, 5, ADJ>(P, a, grid, nwarps, smem, st);
+        default: return rw::dispatch_ck<12, 5, ADJ>(P, a, grid, nwarps, smem, st);
+    }
+}
 }  // namespace
 
 // n_units > 1: a chain of units solved in place in one launch (prepared tables, unit u at w + u * unit_stride)
@@ -180,30 +209,23 @@ int launch_inverse_rw_chain(const float* z, const float* w, float* x, const Shap
     bool planned = false;
     int rc = plan_inverse_rw(z, w, x, s, prepared, n_units, u_first, u_step, unit_stride, plan, &planned);
     if (rc || !planned) return rc;
-    const RwArgs& a = plan.a;
-    const int C = s.C, KS = s.kH, P = plan.P, nwarps = plan.nwarps;
-    const dim3 grid = plan.grid;
-    const size_t smem = plan.smem;
-    if (KS == 3) {
-        switch (C) {
-            case 1: rc = rw::dispatch_ck<1, 3>(P, a, grid, nwarps, smem, st); break;
-            case 2: rc = rw::dispatch_ck<2, 3>(P, a, grid, nwarps, smem, st); break;
-            case 3: rc = rw::dispatch_ck<3, 3>(P, a, grid, nwarps, smem, st); break;
-            case 4: rc = rw::dispatch_ck<4, 3>(P, a, grid, nwarps, smem, st); break;
-            case 6: rc = rw::dispatch_ck<6, 3>(P, a, grid, nwarps, smem, st); break;
-            default: rc = rw::dispatch_ck<12, 3>(P, a, grid, nwarps, smem, st); break;
-        }
-    } else {
-        switch (C) {
-            case 1: rc = rw::dispatch_ck<1, 5>(P, a, grid, nwarps, smem, st); break;
-            case 2: rc = rw::dispatch_ck<2, 5>(P, a, grid, nwarps, smem, st); break;
-            case 3: rc = rw::dispatch_ck<3, 5>(P, a, grid, nwarps, smem, st); break;
-            case 4: rc = rw::dispatch_ck<4, 5>(P, a, grid, nwarps, smem, st); break;
-            case 6: rc = rw::dispatch_ck<6, 5>(P, a, grid, nwarps, smem, st); break;
-            default: rc = rw::dispatch_ck<12, 5>(P, a, grid, nwarps, smem, st); break;
-        }
-    }
+    rc = dispatch_plan<false>(plan, s, st);
     if (rc == FINC_E_UNSUPPORTED) return prepared ? FINC_E_UNSUPPORTED : 0;
+    *handled = true;
+    return rc;
+}
+
+// The adjoint solve dz = A^-T dx (`s.orders` already flipped by the caller): the launch the inverse of the same shape
+// would make -- same plan, same P, NSTK, T -- of the ADJ instantiation.  *handled = false when the shape is not covered.
+int launch_inverse_rw_adjoint(const float* dx, const float* w, float* dz, const Shape& s, cudaStream_t st,
+                              bool* handled) {
+    *handled = false;
+    RwPlan plan;
+    bool planned = false;
+    int rc = plan_inverse_rw(dx, w, dz, s, false, 1, 0, 1, 0, plan, &planned);
+    if (rc || !planned) return rc;
+    rc = dispatch_plan<true>(plan, s, st);
+    if (rc == FINC_E_UNSUPPORTED) return 0;
     *handled = true;
     return rc;
 }

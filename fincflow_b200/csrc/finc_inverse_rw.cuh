@@ -25,6 +25,12 @@
 //     eight 4x4x12 tiles fill a warp with no reduction at all.
 //   * weights: registers when C*C/P*(KH*KW-1) is small (sign folded in), else 128-bit broadcast
 //     loads from the sweep-ordered table (same table as finc_inverse_wave.cuh).
+//   * ADJ = true solves the adjoint system A^T g = dx of the same map instead (the input gradient of the
+//     inverse, finc_inverse_adjoint_f32).  A^T is itself a FInC inverse, swept from the opposite corner
+//     (the host flips every group's order) with the weights w''[o, i, a, b] = w[C-1-i, C-1-o, kH-1-a, kW-1-b]
+//     and the channels reversed on the way in and out.  The staging builds the sweep-ordered table of w''
+//     straight from the raw weights and the channel reversal lives in compile-time register indices, so the
+//     recurrence, the data movement and the register budget are those of the inverse.
 #pragma once
 #include "finc_inverse_wave.cuh"
 
@@ -77,7 +83,7 @@ struct Cfg {
 // has to be cleared at a tile top and the row pointer never wraps, which shortens the step.
 // WREG / CREG: tap / corner weights held in registers (sign folded in) instead of read from the shared-memory table;
 // x * (-w) and (-x) * w round identically, so both give the same bits.
-template <int C, int KH, int KW, int P, bool MT, bool WREG, bool CREG>
+template <int C, int KH, int KW, int P, bool MT, bool WREG, bool CREG, bool ADJ>
 __device__ __forceinline__ void inverse_rw_body(const RwArgs& a, int vblock, int vgrid, int grp) {
     using K = Cfg<C, KH, KW, P>;
     constexpr int CL = K::CL;
@@ -91,6 +97,11 @@ __device__ __forceinline__ void inverse_rw_body(const RwArgs& a, int vblock, int
     const Shape& s = a.s;
     const int H = s.H, W = s.W;
     const int HW = H * W;
+    // channel c of the solved system is channel rv(c) of z and x.  The adjoint reverses the channels in the register
+    // indices only (all compile-time), so its shared-memory addressing and register allocation are the inverse's:
+    // lane p's window entry il holds system channel rv(il*P + p), and row r of the weight table belongs to system
+    // input channel rv(r).  (Reversing them in the addresses instead cost the C = 12, 5x5 kernel spills.)
+    auto rv = [](int c) -> int { return ADJ ? C - 1 - c : c; };
     const int NSTK = a.NSTK;
     const int item_tiles = NSTK * a.T;
     const int stage_floats = NSTK * a.stack_stride;
@@ -162,10 +173,18 @@ __device__ __forceinline__ void inverse_rw_body(const RwArgs& a, int vblock, int
             r /= KW;
             const int aa = r % KH;
             r /= KH;
-            const int i = r % C, o = r / C;
+            int i = r % C, o = r / C;
+            int ta = aa, tb = b;
+            if constexpr (ADJ) {   // raw w[o][i][aa][b] is w''[C-1-i][C-1-o][KH-1-aa][KW-1-b], in table row rv(C-1-o) = o
+                const int o2 = C - 1 - i;
+                i = o;
+                o = o2;
+                ta = KH - 1 - aa;
+                tb = KW - 1 - b;
+            }
             const int ord = order_of(s.orders, g);
-            const int kh = (ord & 2) ? aa : KH - 1 - aa;
-            const int kw = (ord & 1) ? b : KW - 1 - b;
+            const int kh = (ord & 2) ? ta : KH - 1 - ta;
+            const int kw = (ord & 1) ? tb : KW - 1 - tb;
             wk[((gl * KH + kh) * KW + kw) * TS + i * CPP + o] = v;
         });
         __syncthreads();
@@ -219,7 +238,7 @@ __device__ __forceinline__ void inverse_rw_body(const RwArgs& a, int vblock, int
 #pragma unroll
             for (int i = 0; i < C; ++i)
 #pragma unroll
-                for (int o = 0; o < C; ++o) wc[i][o] = wg[i * CPP + o];
+                for (int o = 0; o < C; ++o) wc[i][o] = wg[rv(i) * CPP + o];
         }
 
         // this lane's stack
@@ -243,7 +262,7 @@ __device__ __forceinline__ void inverse_rw_body(const RwArgs& a, int vblock, int
                 for (int il = 0; il < CL; ++il) win[kw][kh][il] = 0.f;
         float zc[C];   // z of the pixel solved in the current step (loaded one step ahead)
 #pragma unroll
-        for (int o = 0; o < C; ++o) zc[o] = (s_begin == 0 && s_end > 0 && p == 0) ? ptr[o * HW] : 0.f;
+        for (int o = 0; o < C; ++o) zc[rv(o)] = (s_begin == 0 && s_end > 0 && p == 0) ? ptr[o * HW] : 0.f;
 
         for (int step0 = 0; step0 < nsteps; step0 += KH) {
 #pragma unroll
@@ -272,7 +291,7 @@ __device__ __forceinline__ void inverse_rw_body(const RwArgs& a, int vblock, int
                 const bool act_n = step + 1 >= s_begin && step + 1 < s_end;
                 float zn[C];
 #pragma unroll
-                for (int o = 0; o < C; ++o) zn[o] = (act_n && p == 0) ? nptr[o * HW] : 0.f;
+                for (int o = 0; o < C; ++o) zn[rv(o)] = (act_n && p == 0) ? nptr[o * HW] : 0.f;
                 // (3) first row of a tile: nothing above it (the zero padding of the reference)
                 if constexpr (MT) {
                     if (hn == 0) {
@@ -342,7 +361,7 @@ __device__ __forceinline__ void inverse_rw_body(const RwArgs& a, int vblock, int
                     } else if constexpr (CPP % 4 == 0) {
 #pragma unroll
                         for (int v = (i + 1) / 4; v < CPP / 4; ++v) {
-                            const float4 f = *reinterpret_cast<const float4*>(wg + i * CPP + 4 * v);
+                            const float4 f = *reinterpret_cast<const float4*>(wg + rv(i) * CPP + 4 * v);
                             if (4 * v + 0 > i && 4 * v + 0 < C) acc[4 * v + 0] = fmaf(-acc[i], f.x, acc[4 * v + 0]);
                             if (4 * v + 1 > i && 4 * v + 1 < C) acc[4 * v + 1] = fmaf(-acc[i], f.y, acc[4 * v + 1]);
                             if (4 * v + 2 > i && 4 * v + 2 < C) acc[4 * v + 2] = fmaf(-acc[i], f.z, acc[4 * v + 2]);
@@ -350,15 +369,15 @@ __device__ __forceinline__ void inverse_rw_body(const RwArgs& a, int vblock, int
                         }
                     } else {
 #pragma unroll
-                        for (int o = i + 1; o < C; ++o) acc[o] = fmaf(-acc[i], wg[i * CPP + o], acc[o]);
+                        for (int o = i + 1; o < C; ++o) acc[o] = fmaf(-acc[i], wg[rv(i) * CPP + o], acc[o]);
                     }
                 }
                 // (8) keep this lane's channels in the window; one lane per channel stores
 #pragma unroll
                 for (int il = 0; il < CL; ++il) {
-                    float v = acc[il * P];
+                    float v = acc[rv(il * P)];
 #pragma unroll
-                    for (int pp = 1; pp < P; ++pp) v = (p == pp) ? acc[il * P + pp] : v;
+                    for (int pp = 1; pp < P; ++pp) v = (p == pp) ? acc[rv(il * P + pp)] : v;
                     win[0][ph][il] = v;
                     if (active) ptr[(il * P + p) * HW] = v;
                 }
@@ -399,10 +418,16 @@ __device__ __forceinline__ void inverse_rw_body(const RwArgs& a, int vblock, int
     if (threadIdx.x == 0) dbg_mark(a.dbg, 4);
 }
 
-template <int C, int KH, int KW, int P, bool MT>
+// the corner weights of the C = 12, P = 1 single-tile adjoint come from the shared-memory table: held in registers
+// they spill (24 B; the inverse of that family spills 20 B and keeps them, as before)
+template <int C, int P, bool MT, bool ADJ>
+constexpr bool creg_of(bool creg) { return creg && !(ADJ && C == 12 && P == 1 && !MT); }
+
+template <int C, int KH, int KW, int P, bool MT, bool ADJ>
 __global__ void __launch_bounds__(Cfg<C, KH, KW, P>::MAXW * 32, 1) inverse_rw_kernel(const RwArgs a) {
     using K = Cfg<C, KH, KW, P>;
-    inverse_rw_body<C, KH, KW, P, MT, K::WREG, K::CREG>(a, (int)blockIdx.x, (int)gridDim.x, (int)blockIdx.y);
+    inverse_rw_body<C, KH, KW, P, MT, K::WREG, creg_of<C, P, MT, ADJ>(K::CREG), ADJ>(
+        a, (int)blockIdx.x, (int)gridDim.x, (int)blockIdx.y);
 }
 
 // ---- several levels in one launch (finc_inverse_chain_multi_f32) ------------------------------------------------
@@ -430,7 +455,7 @@ struct RwKind {
 
 template <class K>
 __device__ __forceinline__ void run_kind(const RwArgs& a, int vblock, int vgrid, int grp) {
-    inverse_rw_body<K::C, K::KS, K::KS, K::P, false, K::WREG, K::CREG>(a, vblock, vgrid, grp);
+    inverse_rw_body<K::C, K::KS, K::KS, K::P, false, K::WREG, K::CREG, false>(a, vblock, vgrid, grp);
 }
 
 template <class K0, class K1, class K2>
@@ -455,15 +480,15 @@ using RwKind2 = RwKind<12, 3, 4, false, false>;
 int launch_multi(const RwMultiArgs& m, int n_ctas, size_t smem, cudaStream_t st);   // finc_inverse_rw_multi.cu
 int multi_ctas_per_sm(size_t smem);   // CTAs of the multi-level kernel one SM holds with `smem` bytes each (0 on error)
 
-template <int C, int KH, int KW, int P>
+template <int C, int KH, int KW, int P, bool ADJ>
 int launch_inst(const RwArgs& a, dim3 grid, int nwarps, size_t smem, cudaStream_t st) {
     if (a.T > 1) {
-        auto kern = inverse_rw_kernel<C, KH, KW, P, true>;
+        auto kern = inverse_rw_kernel<C, KH, KW, P, true, ADJ>;
         cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e != cudaSuccess) return (int)e;
         return launch_kernel(kern, grid, nwarps * 32, smem, st, a);
     }
-    auto kern = inverse_rw_kernel<C, KH, KW, P, false>;
+    auto kern = inverse_rw_kernel<C, KH, KW, P, false, ADJ>;
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return (int)e;
     return launch_kernel(kern, grid, nwarps * 32, smem, st, a);
@@ -487,19 +512,20 @@ constexpr int rw_max_warps(int C, int KH, int KW, int P) {
     return EST <= 100 ? 16 : 8;
 }
 
-template <int C, int KH, int KW>
+template <int C, int KH, int KW, bool ADJ>
 int dispatch_p(int P, const RwArgs& a, dim3 grid, int nwarps, size_t smem, cudaStream_t st) {
-    if constexpr (rw_supported(C, KH, KW, 1)) { if (P == 1) return launch_inst<C, KH, KW, 1>(a, grid, nwarps, smem, st); }
-    if constexpr (rw_supported(C, KH, KW, 2)) { if (P == 2) return launch_inst<C, KH, KW, 2>(a, grid, nwarps, smem, st); }
-    if constexpr (rw_supported(C, KH, KW, 4)) { if (P == 4) return launch_inst<C, KH, KW, 4>(a, grid, nwarps, smem, st); }
-    if constexpr (rw_supported(C, KH, KW, 8)) { if (P == 8) return launch_inst<C, KH, KW, 8>(a, grid, nwarps, smem, st); }
+    if constexpr (rw_supported(C, KH, KW, 1)) { if (P == 1) return launch_inst<C, KH, KW, 1, ADJ>(a, grid, nwarps, smem, st); }
+    if constexpr (rw_supported(C, KH, KW, 2)) { if (P == 2) return launch_inst<C, KH, KW, 2, ADJ>(a, grid, nwarps, smem, st); }
+    if constexpr (rw_supported(C, KH, KW, 4)) { if (P == 4) return launch_inst<C, KH, KW, 4, ADJ>(a, grid, nwarps, smem, st); }
+    if constexpr (rw_supported(C, KH, KW, 8)) { if (P == 8) return launch_inst<C, KH, KW, 8, ADJ>(a, grid, nwarps, smem, st); }
     return FINC_E_UNSUPPORTED;
 }
 
-// explicitly instantiated in finc_inverse_rw_c<N>k<K>.cu so the instantiations compile in parallel
-template <int C, int KS>
+// explicitly instantiated in finc_inverse_rw_c<N>k<K>.cu (inverse) and finc_inverse_rw_adj_c<N>k<K>.cu (adjoint)
+// so the instantiations compile in parallel
+template <int C, int KS, bool ADJ = false>
 int dispatch_ck(int P, const RwArgs& a, dim3 grid, int nwarps, size_t smem, cudaStream_t st) {
-    return dispatch_p<C, KS, KS>(P, a, grid, nwarps, smem, st);
+    return dispatch_p<C, KS, KS, ADJ>(P, a, grid, nwarps, smem, st);
 }
 
 }  // namespace rw

@@ -1,0 +1,7 @@
+// explicit instantiation of the register-window adjoint solve (finc_inverse_adjoint_f32) for C = 6, 3x3 kernels
+#include "finc_inverse_rw.cuh"
+namespace finc {
+namespace rw {
+template int dispatch_ck<6, 3, true>(int, const RwArgs&, dim3, int, size_t, cudaStream_t);
+}
+}

@@ -44,6 +44,9 @@ __global__ void conv_naive_kernel(const float* __restrict__ x, const float* __re
 // one CTA per tile (n,g); anti-diagonal wavefront with two block barriers per diagonal,
 // operating in place on the output in global memory.
 // reference: utils/fastflow_cuda_inverse/cinc_cuda_kernel_level2.cu:49-72,98-132.
+// ADJ: the adjoint solve of finc_inverse_adjoint_f32 -- the same sweep with `s.orders` flipped by the host, the
+// weights w''[o][i][a][b] = w[C-1-i][C-1-o][kH-1-a][kW-1-b] and channel c of the system at channel C-1-c.
+template <bool ADJ>
 __global__ void inverse_naive_kernel(const float* z, const float* __restrict__ w, float* x, Shape s) {
     const long HW = (long)s.H * s.W;
     const int H = s.H, W = s.W, C = s.C, kH = s.kH, kW = s.kW;
@@ -55,6 +58,11 @@ __global__ void inverse_naive_kernel(const float* z, const float* __restrict__ w
         volatile float* xt = x + tile * C * HW;
         const float* wg = w + (long)g * C * C * kH * kW;
         const int ca = corner_a(ord, kH), cb = corner_b(ord, kW);
+        auto wt = [&](int o, int i, int a, int b) -> float {
+            return ADJ ? wg[(((C - 1 - i) * C + (C - 1 - o)) * kH + (kH - 1 - a)) * kW + (kW - 1 - b)]
+                       : wg[((o * C + i) * kH + a) * kW + b];
+        };
+        auto ch = [&](int c) -> int { return ADJ ? C - 1 - c : c; };
         for (int d = 0; d < H + W - 1; ++d) {
             const int hs_lo = max(0, d - (W - 1));
             const int hs_hi = min(H - 1, d);
@@ -64,7 +72,7 @@ __global__ void inverse_naive_kernel(const float* z, const float* __restrict__ w
                 const int o = it % C;
                 const int hs = hs_lo + it / C, ws = d - hs;
                 const int h = bot ? H - 1 - hs : hs, ww = right ? W - 1 - ws : ws;
-                float acc = zt[o * HW + h * W + ww];
+                float acc = zt[ch(o) * HW + h * W + ww];
                 for (int k_h = 0; k_h < kH && k_h <= hs; ++k_h) {
                     const int hh = bot ? h + k_h : h - k_h;
                     const int a = bot ? k_h : kH - 1 - k_h;
@@ -73,10 +81,10 @@ __global__ void inverse_naive_kernel(const float* z, const float* __restrict__ w
                         const int wc = right ? ww + k_w : ww - k_w;
                         const int b = right ? k_w : kW - 1 - k_w;
                         for (int i = 0; i < C; ++i)
-                            acc = fmaf(-xt[i * HW + hh * W + wc], wg[((o * C + i) * kH + a) * kW + b], acc);
+                            acc = fmaf(-xt[ch(i) * HW + hh * W + wc], wt(o, i, a, b), acc);
                     }
                 }
-                xt[o * HW + h * W + ww] = acc;
+                xt[ch(o) * HW + h * W + ww] = acc;
             }
             __syncthreads();
             // phase B: channel-triangular corner tap, sequential in o inside one thread
@@ -84,10 +92,10 @@ __global__ void inverse_naive_kernel(const float* z, const float* __restrict__ w
                 const int hs = hs_lo + p, ws = d - hs;
                 const int h = bot ? H - 1 - hs : hs, ww = right ? W - 1 - ws : ws;
                 for (int o = 1; o < C; ++o) {
-                    float acc = xt[o * HW + h * W + ww];
+                    float acc = xt[ch(o) * HW + h * W + ww];
                     for (int i = 0; i < o; ++i)
-                        acc = fmaf(-xt[i * HW + h * W + ww], wg[((o * C + i) * kH + ca) * kW + cb], acc);
-                    xt[o * HW + h * W + ww] = acc;
+                        acc = fmaf(-xt[ch(i) * HW + h * W + ww], wt(o, i, ca, cb), acc);
+                    xt[ch(o) * HW + h * W + ww] = acc;
                 }
             }
             __syncthreads();
@@ -126,6 +134,7 @@ __global__ void wgrad_naive_kernel(const float* __restrict__ dz, const float* __
         if (lane == 0) {
             const bool masked = !(flags & FINC_FLAG_NO_MASK) && a == corner_a(ord, s.kH) && b == corner_b(ord, s.kW) && i >= o;
             if (masked) acc = 0.f;
+            else if (flags & FINC_FLAG_NEGATE) acc = -acc;
             if (flags & FINC_FLAG_ACCUMULATE) acc += dw[e];
             dw[e] = acc;
         }
@@ -264,7 +273,13 @@ int launch_conv_naive(const float* x, const float* w, float* y, const Shape& s, 
 
 int launch_inverse_naive(const float* z, const float* w, float* x, const Shape& s, cudaStream_t st) {
     const long tiles = (long)s.B * s.G;
-    inverse_naive_kernel<<<(unsigned)(tiles > 148L * 32 ? 148L * 32 : tiles), 128, 0, st>>>(z, w, x, s);
+    inverse_naive_kernel<false><<<(unsigned)(tiles > 148L * 32 ? 148L * 32 : tiles), 128, 0, st>>>(z, w, x, s);
+    return (int)cudaGetLastError();
+}
+
+int launch_inverse_adjoint_naive(const float* dx, const float* w, float* dz, const Shape& s, cudaStream_t st) {
+    const long tiles = (long)s.B * s.G;
+    inverse_naive_kernel<true><<<(unsigned)(tiles > 148L * 32 ? 148L * 32 : tiles), 128, 0, st>>>(dx, w, dz, s);
     return (int)cudaGetLastError();
 }
 

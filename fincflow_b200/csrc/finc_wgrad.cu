@@ -310,6 +310,7 @@ __global__ void __launch_bounds__((max_consumer_warps(OB, KH) + 1) * 32, 1) wgra
         const int ab = idx % (KH * KW);
         const long out = (((long)g * C + o) * C + i) * KH * KW + ab;
         if (!(a.flags & FINC_FLAG_NO_MASK) && ab == ca * KW + cbn && i >= o) v = 0.f;
+        else if (a.flags & FINC_FLAG_NEGATE) v = -v;
         if (a.flags & FINC_FLAG_ACCUMULATE) v += dw_u[out];
         dw_u[out] = v;
     };

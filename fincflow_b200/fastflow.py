@@ -5,7 +5,8 @@ Drop-in for the reference's fastflow/fastflow.py:13-100: same constructor
 in_channels % 4 == 0), same sub-module names (`conv_tl/tr/bl/br`, each exposing
 `.conv.weight`, `.mask`, `.order`, `reset_gradients()`), same state-dict keys
 (`conv_tl.conv.weight`, ...), `forward(x, context=None) -> (out, logdet)`,
-`reverse(x, context=None) -> out` (bare tensor, fastflow.py:100).
+`reverse(x, context=None) -> out` (bare tensor, fastflow.py:100; differentiable, which the reference's reverse is not: see
+ops.finc_inverse).
 
 B200-first differences (results identical):
   * the four weights live in ONE packed parameter `weight` [4*Cq, Cq, kH, kW] in their
@@ -125,7 +126,10 @@ class FastFlowUnit(nn.Module):
     def reverse(self, x, context=None):
         if (self.dense_reverse and x.is_cuda and not (torch.is_grad_enabled() and x.requires_grad)
                 and _native.inverse_dense_bytes(4, self.cq, x.shape[2], x.shape[3]) > 0):
-            return _native.inverse_dense(x.contiguous(), self._dense_table(int(x.shape[2]), int(x.shape[3])))
+            # (a graph for the weight alone -- weight_grad_in_reverse -- keeps the dense forward; its backward is the
+            # adjoint wavefront)
+            return finc_inverse(x, self.weight, 4, _native.ORDERS_UNIT,
+                                dense=self._dense_table(int(x.shape[2]), int(x.shape[3])))
         return finc_inverse(x, self.weight, 4, _native.ORDERS_UNIT)
 
     def logdet(self, x, context=None):

@@ -27,6 +27,7 @@ import torch.nn.functional as F
 
 from . import _native
 from .fastflow import FastFlowUnit
+from .ops import reverse_records
 from .layers.flowlayer import FlowLayer, PreprocessingFlowLayer
 
 
@@ -398,10 +399,12 @@ class Preprocess(nn.Module):
             logdet = logdet + ld
         return x, logdet
 
-    def reverse(self, x):
-        if self.fused and x.is_cuda and x.dtype == torch.float32 and not torch.is_grad_enabled():
+    def reverse(self, x, quantize=True):
+        """`quantize=False` stops before Dequantization's floor and returns the continuous image in [0, 256), whose
+        gradient reaches the latents and the parameters (the floored image has zero gradient everywhere)."""
+        if quantize and self.fused and x.is_cuda and x.dtype == torch.float32 and not torch.is_grad_enabled():
             return _native.preprocess(x, None, self.alpha, reverse=True)[0]
-        for layer in reversed(self.layers):
+        for layer in reversed(self.layers if quantize else self.layers[1:]):
             x = layer.reverse(x)
         return x
 
@@ -473,6 +476,23 @@ def affine_of(actnorm, conv1x1):
         return W, None
     A = W * torch.exp(-actnorm.log_scale).unsqueeze(0)
     return A, -(A @ actnorm.translation)
+
+
+class _InverseFn(torch.autograd.Function):
+    """W^-1 of one Conv1x1 weight on finc_slogdet_inverse_f32 (the same bits as the cached reverse constants of
+    _glue_constants); backward -W^-T g W^-T"""
+
+    @staticmethod
+    def forward(ctx, W):
+        Winv = _native.slogdet_inverse(W.unsqueeze(0).contiguous())[1][0]
+        ctx.save_for_backward(Winv)
+        return Winv
+
+    @staticmethod
+    def backward(ctx, g):
+        (Winv,) = ctx.saved_tensors
+        WinvT = Winv.t()
+        return -(WinvT @ g @ WinvT)
 
 
 class _SlogdetFn(torch.autograd.Function):
@@ -554,6 +574,13 @@ def _fused_glow_reverse(self, z):
     act = getattr(gs, "actnorm", None)
     assert act is None or act.is_initialized()
     x = gs.coupling.reverse(z)
+    act_ps = [act.translation, act.log_scale] if act is not None else []
+    if reverse_records(x, gs.conv1x1.W, *act_ps):
+        # differentiable: A^-1 = exp(log_s)[:, None] W^-1 and the bias t, computed as _glue_constants does (same bits)
+        W = gs.conv1x1.W
+        Winv = _InverseFn.apply(W) if W.is_cuda and W.shape[0] <= 128 else torch.inverse(W)
+        Ainv = Winv if act is None else torch.exp(act.log_scale).unsqueeze(1) * Winv
+        return _Affine1x1Fn.apply(x, Ainv, None if act is None else act.translation)
     _, _, _, Ainv, binv = _glue_constants(self)
     return _native.affine1x1(x.contiguous(), Ainv, binv)
 
@@ -673,7 +700,10 @@ class FastFlow(nn.Module):
         zs.append(x)
         return zs, logdet + self.base_distribution.log_prob(x)
 
-    def reverse(self, n_samples=1, zs=None, z_std=1.0):
+    def reverse(self, n_samples=1, zs=None, z_std=1.0, quantize=True):
+        """x = the flow's inverse of the latents `zs` (sampled when None).  Differentiable in `zs` and every parameter
+        the inverse uses (ops.finc_inverse says when a graph is recorded); `quantize=False` returns the continuous image before the final floor, which has zero gradient
+        (Preprocess.reverse)."""
         if zs is None:
             zs = [self.base_distribution.sample(n_samples)[0]]
         z = zs[-1]
@@ -682,7 +712,7 @@ class FastFlow(nn.Module):
         x = self.squeeze.reverse(z)
         for i, level in enumerate(reversed(self.fastflow_levels)):
             x = level.reverse(x) if len(zs) == 1 else level.reverse(x, zs[-i - 2])
-        return self.preprocess.reverse(x)
+        return self.preprocess.reverse(x, quantize=quantize)
 
     def log_prob(self, x, bits_per_pixel=False):
         """bits_per_pixel: per IMAGE dimension (x[0].numel()).  The reference divides by `zs[0].numel()`, a

@@ -25,7 +25,8 @@
  *     legacy default stream) of the calling thread's current CUDA device, allocates
  *     nothing, keeps no state between calls, and returns 0 or a negative FINC_E_* code /
  *     positive cudaError_t.  It never throws.
- *   - outputs must not alias inputs, except finc_inverse_f32 where x == z is allowed.
+ *   - outputs must not alias inputs, except finc_inverse_f32 where x == z is allowed and
+ *     finc_inverse_adjoint_f32 where dz == dx is allowed.
  */
 #ifndef FINCFLOW_B200_H_
 #define FINCFLOW_B200_H_
@@ -57,6 +58,7 @@ extern "C" {
 #define FINC_FLAG_LOGDET_ACCUMULATE 8u /* forward: logdet[n] += ... (FlowSequential's `logdet += layer_logdet`) */
 #define FINC_FLAG_TF32_1PASS 1024u /* tensor-core entry points: single-pass TF32 products (PyTorch's default conv precision, ~5e-4) instead of the fp32-accurate 3xTF32 split */
 #define FINC_FLAG_CHAIN_TRANSPOSE 2048u /* finc_chain_f32: backward-data chain (transposed weights, opposite corner) */
+#define FINC_FLAG_NEGATE 4096u /* backward_weight (and _batched): dw = -result (dw += -result with FINC_FLAG_ACCUMULATE); masked entries stay +0 */
 
 /* error codes (negative); positive return values are cudaError_t */
 #define FINC_OK 0
@@ -117,6 +119,20 @@ int finc_backward_weight_f32(const float* dz, const float* x, float* dw,
 int finc_inverse_f32(const float* z, const float* w, float* x,
                      int B, int G, int C, int H, int W, int kH, int kW,
                      unsigned orders, unsigned flags, void* stream);
+
+/* The exact adjoint (transpose) of finc_inverse_f32 -- the input gradient of the sampling direction: with
+ * A the map finc_inverse_f32 inverts (x = A^-1 z), dz = A^-T dx, i.e. <dx, inverse(z)> = <adjoint(dx), z> for all z.
+ * Equivalently finc_backward_input_f32(dz) == dx.  With autograd this gives, for x = inverse(z; w) and an upstream
+ * gradient dx:  dL/dz = dz  and  dL/dw = -(finc_backward_weight_f32(dz, x), masked), i.e. one call of
+ * finc_backward_weight_f32 with FINC_FLAG_NEGATE (the inverse never reads w[o, i>=o, a*, b*], so their derivative
+ * is 0 whatever the mask setting of the forward layer).
+ * It is a FInC inverse in its own right, swept from the opposite corner of every group; one launch, same kernels and
+ * cost as finc_inverse_f32 of the same shape (register-window kernel where that covers the shape, the generic
+ * kernel otherwise).  Arguments as finc_inverse_f32; dz == dx is allowed; B = 0 is a no-op.  flags: FINC_FLAG_NAIVE
+ * forces the generic kernel (testing); FINC_FLAG_PREPARED is not supported (FINC_E_UNSUPPORTED). */
+int finc_inverse_adjoint_f32(const float* dx, const float* w, float* dz,
+                             int B, int G, int C, int H, int W, int kH, int kW,
+                             unsigned orders, unsigned flags, void* stream);
 
 /* dw[gC+o, i, a*_g, b*_g] = 0 for i >= o.  Replaces PaddedConv2d.reset_gradients
  * (layers/conv.py:98-99: H2D copy of the CPU mask + multiply). */
