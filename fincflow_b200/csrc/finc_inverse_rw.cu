@@ -120,15 +120,26 @@ int plan_inverse_rw(const float* z, const float* w, float* x, const Shape& s, bo
         if (warps >= ctas_max * 4) { P = cand[i]; break; }
     }
     if (C == 6 && KS == 3 && nc > 1 && P == 1) P = 2;  // P = 2 keeps the C = 6 weights in registers
-    P = env_int("FINC_RW_P", P);
+    // FINC_RW_P / _NSTK / _T / _S / _WARPS (experiment and test knobs, read per call) pin parts of the plan; a value
+    // outside what the planner itself could choose is ignored, so a knob never addresses lanes or shared memory the
+    // kernel does not own
+    {
+        const int fp = env_int("FINC_RW_P", 0);
+        for (int i = 0; i < nc; ++i)
+            if (cand[i] == fp) P = fp;
+    }
     // stacks per warp: all 32/(WP*P) lanes groups when the batch can fill the SMs, fewer (idle lanes,
     // more warps) when it cannot
     int NSTK = 32 / (WP * P);
     while (NSTK > 1 && tiles / NSTK < ctas_max * 2) NSTK /= 2;   // (x4 was measured slower at batch 256)
-    NSTK = env_int("FINC_RW_NSTK", NSTK);
+    {
+        const int fn = env_int("FINC_RW_NSTK", 0);   // a power of two whose stacks fit the warp
+        if (fn >= 1 && (fn & (fn - 1)) == 0 && fn * WP * P <= 32) NSTK = fn;
+    }
     a.NSTK = NSTK;
     const int maxw_k = rw::rw_max_warps(C, KS, KS, P);
-    const int maxw = env_int("FINC_RW_WARPS", maxw_k) < maxw_k ? env_int("FINC_RW_WARPS", maxw_k) : maxw_k;
+    const int fw = env_int("FINC_RW_WARPS", 0);
+    const int maxw = (fw >= 1 && fw < maxw_k) ? fw : maxw_k;
 
     const size_t wk_bytes = (size_t)((a.wk_floats + 31) & ~31) * 4 * n_units;
     const size_t avail = budget - wk_bytes;
@@ -144,7 +155,10 @@ int plan_inverse_rw(const float* z, const float* w, float* x, const Shape& s, bo
         if (stage_bytes_of(T2) * maxw + 64 > avail && stage_bytes_of(T2) * 8 + 64 > avail) break;
         T = T2;
     }
-    T = env_int("FINC_RW_T", T);
+    {
+        const int ft = env_int("FINC_RW_T", 0);
+        if (ft == 1 || ft == 2 || ft == 4 || ft == 8) T = ft;
+    }
     a.T = T;
     a.stack_stride = T * a.tile_stride + skew;
     const size_t stage_bytes = stage_bytes_of(T);
@@ -159,7 +173,10 @@ int plan_inverse_rw(const float* z, const float* w, float* x, const Shape& s, bo
     if (nwarps < 1) return prepared ? FINC_E_UNSUPPORTED : 0;
     // a second stage only pays when warps loop over several items and memory is left
     if (items_per_cta > nwarps && (size_t)nwarps * 2 * (stage_bytes + 8) + 64 <= avail) a.S = 2;
-    a.S = env_int("FINC_RW_S", a.S);
+    {
+        const int fs = env_int("FINC_RW_S", 0);
+        if (fs == 1 || fs == 2) a.S = fs;
+    }
     const size_t smem = wk_bytes + (size_t)nwarps * a.S * (stage_bytes + 8) + 8 + 16;
     if (smem > budget + 2048) return prepared ? FINC_E_UNSUPPORTED : 0;
     plan.a = a;
