@@ -38,14 +38,14 @@ int launch_igemm_rows(int BN, int npass, const CUtensorMap& a, const CUtensorMap
     return npass == 1 ? launch_igemm_rows_p1(BN, a, b, g, e, st) : launch_igemm_rows_p3(BN, a, b, g, e, st);
 }
 
-// CTAs per cluster for the channels-last GEMMs: FINC_TC_CLUSTER = 1 | 2 | 4 (experiments); default below
+// CTAs per cluster for the channels-last GEMMs: FINC_TC_CLUSTER = 1 | 2 | 4 (experiments), read on every call like
+// the FInC plan knobs; a size the kernel cannot take is lowered below
 static int cluster_size(int BN, int m_tiles) {
-    static int env = -1;
-    if (env < 0) {
-        const char* v = getenv("FINC_TC_CLUSTER");
-        env = v ? atoi(v) : 0;
-    }
-    int cl = env > 0 ? env : 1;   // measured on B200: 1 and 2 tie (the layer is not L2-bound), 4 loses to the lock-step
+    const char* v = getenv("FINC_TC_CLUSTER");
+    const int env = v ? atoi(v) : 0;
+    int cl = env > 4 ? 4 : env > 0 ? env : 1;   // measured on B200: 1 and 2 tie (the layer is not L2-bound), 4 loses
+    // (more than 4 would pass the divisibility rule at BN = 128 and launch the CL = 1 kernel with a weight box of
+    // BN / cl rows, whose `full` barrier then never completes)
     while (cl > 1 && ((BN / cl) % 8 != 0 || BN % cl != 0 || m_tiles < cl || (BN == 32 && cl == 4))) cl >>= 1;
     return cl;
 }

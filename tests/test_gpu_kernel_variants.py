@@ -47,8 +47,6 @@ FAMILIES = {
     "chain": "finc::chain::chain_kernel",
     "inverse_wave": "finc::wave::inverse_wave_kernel",
 }
-_KERNEL_RE = re.compile("(" + "|".join(re.escape(p) for p in FAMILIES.values()) + r")<([^<>]*)>")
-_FAMILY_OF = {p: f for f, p in FAMILIES.items()}
 
 # compiled instantiations the planners can never select, with the reason (from the code)
 UNREACHABLE = {
@@ -62,32 +60,40 @@ def _arg(v):
     return {"true": 1, "false": 0}[v] if v in ("true", "false") else int(v)
 
 
-def kernels_in(names):
-    """{(family, template arguments)} of the five FInC families among kernel names (bools as 0 / 1)"""
+def kernels_in(names, families=FAMILIES):
+    """{(family, template arguments)} of the kernel families in `families` (name -> qualified template name, by
+    default the five FInC families) among kernel names (bools as 0 / 1)"""
+    pattern = re.compile("(" + "|".join(re.escape(p) for p in families.values()) + r")<([^<>]*)>")
+    family_of = {p: f for f, p in families.items()}
     found = set()
     for name in names:
-        for prefix, args in _KERNEL_RE.findall(name):
-            found.add((_FAMILY_OF[prefix], tuple(_arg(a) for a in args.split(","))))
+        for prefix, args in pattern.findall(name):
+            found.add((family_of[prefix], tuple(_arg(a) for a in args.split(","))))
     return found
 
 
-def launched(fn):
-    """(fn(), the set of FInC kernel instantiations it launched)"""
+def launched(fn, families=FAMILIES):
+    """(fn(), the set of kernel instantiations of `families` it launched)"""
     from torch.profiler import ProfilerActivity, profile
 
     torch.cuda.synchronize()
-    with profile(activities=[ProfilerActivity.CUDA]) as prof:
+    # a PyTorch kernel first: when the session opens with a new CUPTI activity buffer ("Activity Buffer Request"), a
+    # CUDA-only profile of a lone kernel was seen to lose that kernel's record; with CPU activities and a warm-up
+    # kernel ahead of it, it was recorded
+    with profile(activities=[ProfilerActivity.CPU, ProfilerActivity.CUDA]) as prof:
+        torch.zeros(1, device="cuda").add_(1)
+        torch.cuda.synchronize()
         out = fn()
         torch.cuda.synchronize()
-    return out, kernels_in(e.key for e in prof.key_averages())
+    return out, kernels_in((e.key for e in prof.key_averages()), families)
 
 
-def compiled_instantiations():
-    """the instantiations of the five families in the library's symbol table (their host stubs)"""
+def compiled_instantiations(families=FAMILIES):
+    """the instantiations of `families` in the library's symbol table (their host stubs)"""
     from fincflow_b200 import _native
 
     syms = subprocess.run(["nm", "-C", _native.LIB_PATH], capture_output=True, text=True, check=True).stdout
-    return kernels_in(syms.splitlines())
+    return kernels_in(syms.splitlines(), families)
 
 
 @pytest.fixture(scope="module")
