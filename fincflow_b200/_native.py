@@ -31,6 +31,7 @@ FLAG_HALF_GPU = 256
 FLAG_WAVE_SMEM = 512
 FLAG_TF32_1PASS = 1024
 FLAG_NEGATE = 4096
+FLAG_COUPLING_REVERSE = 8192
 PREP_FORWARD, PREP_BACKWARD_INPUT, PREP_INVERSE = 0, 1, 2
 
 # every symbol declared in include/fincflow_b200.h
@@ -571,7 +572,9 @@ def _shared_scratch(nbytes, device):
 
 
 def coupling_backward(x, dy, dlogdet, blob, fwd_workspace, width, flags=0):
-    """(dx, dw1, db1, dw2, db2, dw3, db3, dlogs3) of coupling_apply(forward); `blob` prepared with_backward"""
+    """(dx, dw1, db1, dw2, db2, dw3, db3, dlogs3) of the coupling_apply call that filled `fwd_workspace` from input `x`;
+    `blob` prepared with_backward.  flags | FLAG_COUPLING_REVERSE: that call was a reverse (reverse=True), and `dlogdet`
+    is the gradient of its log-det."""
     x, dy = _prep(x, "x"), _prep(dy, "dy")
     _bind_device(x)
     B, C, H, W = (int(v) for v in x.shape)
@@ -594,8 +597,10 @@ def coupling_backward(x, dy, dlogdet, blob, fwd_workspace, width, flags=0):
     return dx, dw1, db1, dw2, db2, dw3, db3, dlogs3
 
 
-def coupling_apply(x, blob, width, reverse=False, want_logdet=True, logdet_out=None, flags=0, out=None, workspace=None):
-    """Coupling.forward / .reverse (layers/coupling.py:85-99): y, logdet[B] (None for reverse)"""
+def coupling_apply(x, blob, width, reverse=False, want_logdet=None, logdet_out=None, flags=0, out=None, workspace=None):
+    """Coupling.forward / .reverse (layers/coupling.py:85-99): y, logdet[B] or None.  The log-det is the direction's own
+    (reverse: -sum log_s); by default it is computed for the forward and not for the reverse (want_logdet=True or
+    `logdet_out` asks for it)."""
     x = _prep(x, "x")
     _bind_device(x)
     B, C, H, W = (int(v) for v in x.shape)
@@ -605,7 +610,9 @@ def coupling_apply(x, blob, width, reverse=False, want_logdet=True, logdet_out=N
         raise FincNativeError(f"coupling_apply: shape {tuple(x.shape)}, width {width} not covered")
     ws = torch.empty(nbytes, dtype=torch.uint8, device=x.device) if workspace is None else workspace
     logdet = None
-    if not reverse and (want_logdet or logdet_out is not None):
+    if want_logdet is None:
+        want_logdet = not reverse
+    if want_logdet or logdet_out is not None:
         logdet = torch.empty(B, dtype=torch.float32, device=x.device) if logdet_out is None else logdet_out
     _check(load().finc_coupling_apply_f32(x.data_ptr(), y.data_ptr(), None if logdet is None else logdet.data_ptr(),
                                           blob.data_ptr(), ws.data_ptr(), ws.numel(), B, C, H, W, width, int(reverse),

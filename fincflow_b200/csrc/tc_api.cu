@@ -205,6 +205,7 @@ __global__ void rowsum_reduce_kernel(const float* __restrict__ rowsum, float* __
 // every pixel gathers its nine neighbours' tap columns, h[n] = sum_tap Y[pixel + offset(tap), tap, n],
 // and applies the coupling (layers/coupling.py:73-99): h = (h + bias) * exp(3 logs),
 // log_s = 2 tanh(h[2j] / 2), t = h[2j+1], y2 = x2 * exp(log_s) + t  (reverse: (x2 - t) * exp(-log_s)).
+// rowsum (nullable) gets the pixel's log-det term: sum_j log_s, or -sum_j log_s in reverse.
 __global__ void coupling_gather_kernel(const float* __restrict__ Y, const float* __restrict__ bias,
                                        const float* __restrict__ scale, const float* x, float* y,
                                        float* __restrict__ rowsum, int B, int C, int H, int W, int N3pad, int reverse) {
@@ -246,7 +247,7 @@ __global__ void coupling_gather_kernel(const float* __restrict__ Y, const float*
             y[o1] = x[o1];
         }
     }
-    if (rowsum != nullptr) rowsum[pix] = rs;
+    if (rowsum != nullptr) rowsum[pix] = reverse ? -rs : rs;
 }
 
 // Backward-data forms of the three coupling weights, hi / lo split (part 1 follows part 0):
@@ -286,7 +287,11 @@ __global__ void coupling_bwd_weights_kernel(const float* __restrict__ w1, const 
 
 // Backward of the coupling's pointwise part (thread = pixel).  Recomputes h from the saved tap GEMM output Y
 // (same gather as the forward), then with e = exp(log_s), log_s = 2 tanh(hs / 2):
-//   dx2 = dy2 * e;  dlog_s = dy2 * x2 * e + dlogdet[n];  dhs = dlog_s * (1 - tanh^2(hs / 2));  dt = dy2
+//   forward  (y2 = x2 * e + t, logdet = sum log_s):
+//     dx2 = dy2 * e;   dlog_s = dy2 * x2 * e + dlogdet[n];  dt = dy2
+//   reverse  (y2 = (x2 - t) / e, logdet = -sum log_s; x is the reverse's input):
+//     dx2 = dy2 / e;   dlog_s = -dy2 * y2 - dlogdet[n];     dt = -dy2 / e
+//   dhs = dlog_s * (1 - tanh^2(hs / 2))
 //   G3[pixel, 2j] = dhs * s3[2j],  G3[pixel, 2j+1] = dt * s3[2j+1]      (gradient at the conv output, before bias)
 // and the per-pixel terms of db3 = sum G3 and dlogs3 = factor * sum G3 * (acc + b3) go to `red` [pixel][2 * N3pad]
 // for a fixed-order column sum.  dx1 is initialised with dy1 (the col2im pass adds the network's part).
@@ -294,7 +299,8 @@ __global__ void coupling_bwd_pointwise_kernel(const float* __restrict__ Y, const
                                               const float* __restrict__ scale, const float* __restrict__ x,
                                               const float* __restrict__ dy, const float* __restrict__ dlogdet,
                                               float* __restrict__ dx, float* __restrict__ G3, float* __restrict__ red,
-                                              int B, int C, int H, int W, int N3pad, const float* __restrict__ header) {
+                                              int B, int C, int H, int W, int N3pad, const float* __restrict__ header,
+                                              int reverse) {
     const float factor = __ldg(header);   // logscale_factor of the last conv, written by finc_coupling_prepare_f32
     const long np = (long)B * H * W;
     const long pix = blockIdx.x * (long)blockDim.x + threadIdx.x;
@@ -330,14 +336,24 @@ __global__ void coupling_bwd_pointwise_kernel(const float* __restrict__ Y, const
             at = tt + __ldg(bias + 2 * jc + 1);
             const float s0 = __ldg(scale + 2 * jc), s1 = __ldg(scale + 2 * jc + 1);
             const float th = tanhf(as * s0 * 0.5f);
-            const float e = expf(2.0f * th);
             const size_t o2 = base + (size_t)(half + jc) * plane, o1 = base + (size_t)jc * plane;
             const float d2 = dy[o2], x2 = x[o2];
-            dx[o2] = d2 * e;
-            dx[o1] = dy[o1];
-            const float dlog_s = d2 * x2 * e + dld;
+            float dlog_s;
+            if (reverse) {
+                const float ei = expf(-2.0f * th);
+                const float y2 = (x2 - at * s1) * ei;
+                dx[o2] = d2 * ei;
+                dx[o1] = dy[o1];
+                dlog_s = -d2 * y2 - dld;
+                gt = -d2 * ei * s1;
+            } else {
+                const float e = expf(2.0f * th);
+                dx[o2] = d2 * e;
+                dx[o1] = dy[o1];
+                dlog_s = d2 * x2 * e + dld;
+                gt = d2 * s1;
+            }
             gs = dlog_s * (1.f - th * th) * s0;
-            gt = d2 * s1;
         }
         g3[2 * jc] = gs;
         g3[2 * jc + 1] = gt;
@@ -708,7 +724,7 @@ int finc_coupling_apply_f32(const float* x, float* y, float* logdet, const void*
     rc = launch_igemm_rows(BN, npass, mA, mB, g, e, st);
     if (rc) return rc;
     // ... then the nine-neighbour gather + coupling math
-    float* rowsum = (logdet != nullptr && !reverse) ? wsp + ws.rowsum : nullptr;
+    float* rowsum = logdet != nullptr ? wsp + ws.rowsum : nullptr;
     coupling_gather_kernel<<<(unsigned)((np + 127) / 128), 128, 0, st>>>(wsp + ws.y3, p + L.b3, p + L.s3, x, y, rowsum, B,
                                                                         C, H, W, L.N3pad, reverse);
     rc = (int)cudaGetLastError();
@@ -776,9 +792,11 @@ int finc_coupling_backward_f32(const float* x, const float* dy, const float* dlo
     const float* h2 = fws + fw.h2;
     const float* Y = fws + fw.y3;
 
-    // 1. pointwise part: dx2, dx1 = dy1, gradient at the last conv's output, per-pixel terms of db3 / dlogs3
-    coupling_bwd_pointwise_kernel<<<(unsigned)((np + 127) / 128), 128, 0, st>>>(Y, p + L.b3, p + L.s3, x, dy, dlogdet, dx,
-                                                                               s + sc.g3, s + sc.red, B, C, H, W, L.N3pad, p);
+    // 1. pointwise part: dx2, dx1 = dy1, gradient at the last conv's output, per-pixel terms of db3 / dlogs3 (the only
+    //    step that depends on the direction: the network h = net(x1) is the same in both)
+    coupling_bwd_pointwise_kernel<<<(unsigned)((np + 127) / 128), 128, 0, st>>>(
+        Y, p + L.b3, p + L.s3, x, dy, dlogdet, dx, s + sc.g3, s + sc.red, B, C, H, W, L.N3pad, p,
+        (flags & FINC_FLAG_COUPLING_REVERSE) ? 1 : 0);
     int rc = colsum(s + sc.red, s + sc.wcat, s + sc.part, np, 2 * L.N3pad, 2 * L.N3pad, st);
     if (rc) return rc;
     cudaMemcpyAsync(db3, s + sc.wcat, C * sizeof(float), cudaMemcpyDeviceToDevice, st);

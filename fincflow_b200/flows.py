@@ -270,11 +270,26 @@ class Coupling(FlowLayer):
         x1, x2, log_s, t = self._st(input)
         return torch.cat([x1, x2 * torch.exp(log_s) + t], dim=1), log_s.flatten(start_dim=1).sum(-1)
 
+    def _reverse_formulas(self, x):
+        x1, x2, log_s, t = self._st(x)
+        return torch.cat([x1, (x2 - t) * torch.exp(-log_s)], dim=1), -log_s.flatten(start_dim=1).sum(-1)
+
+    def _reverse(self, input, want_logdet):
+        if self._use_tc(input):
+            # a graph exactly when the formulas below would record one
+            if torch.is_grad_enabled() and (input.requires_grad or any(p.requires_grad for p in self._params())):
+                return _CouplingReverseFn.apply(input, self, want_logdet, *self._params())
+            return _native.coupling_apply(input, self.prepared(), self.width, reverse=True, want_logdet=want_logdet,
+                                          flags=self._flags())
+        y, ld = self._reverse_formulas(input)
+        return y, (ld if want_logdet else None)
+
     def reverse(self, input, context=None):
-        if self._use_tc(input) and not torch.is_grad_enabled():
-            return _native.coupling_apply(input, self.prepared(), self.width, reverse=True, flags=self._flags())[0]
-        x1, x2, log_s, t = self._st(input)
-        return torch.cat([x1, (x2 - t) * torch.exp(-log_s)], dim=1)
+        return self._reverse(input, False)[0]
+
+    def reverse_and_logdet(self, input):
+        """(reverse(input), log|det| of the reverse map [B]) = (x, -sum log_s): minus the forward's log-det at x"""
+        return self._reverse(input, True)
 
     def logdet(self, input, context=None):
         return self.forward(input, context)[1]
@@ -325,6 +340,54 @@ class _CouplingFn(torch.autograd.Function):
         return (dx, None, *dps)
 
 
+class _CouplingReverseFn(torch.autograd.Function):
+    """Coupling.reverse (and its log-det -sum log_s when `want_logdet`) with its backward on the tensor-core kernels:
+    finc_coupling_apply_f32(reverse = 1), then one finc_coupling_backward_f32 with FINC_FLAG_COUPLING_REVERSE on the
+    kept workspace.  Widths the backward kernels do not cover (width % 128 != 0) recompute through the PyTorch
+    formulas instead, as _CouplingFn does."""
+
+    @staticmethod
+    def forward(ctx, x, module, want_logdet, *params):
+        ctx.module = module
+        B, C, H, W = x.shape
+        ctx.native = _native.coupling_prepared_bytes(C, module.width, True) > 0
+        ws = None
+        if ctx.native:
+            ws = torch.empty(_native.coupling_workspace_bytes(B, C, H, W, module.width), dtype=torch.uint8, device=x.device)
+        blob = module.prepared(with_backward=ctx.native, training=True)
+        y, logdet = _native.coupling_apply(x, blob, module.width, reverse=True, want_logdet=want_logdet,
+                                           flags=module._flags(), workspace=ws)
+        ctx.save_for_backward(x)
+        ctx.ws, ctx.blob = ws, blob
+        return y, logdet
+
+    @staticmethod
+    def backward(ctx, dy, dlogdet):
+        (x,) = ctx.saved_tensors
+        m = ctx.module
+        if ctx.native:
+            if dy is None:
+                dy = torch.zeros_like(x)
+            grads = _native.coupling_backward(x, dy.contiguous(), dlogdet, ctx.blob, ctx.ws, m.width,
+                                              flags=m._flags() | _native.FLAG_COUPLING_REVERSE)
+            ctx.ws = None
+            return (grads[0], None, None, *grads[1:])
+        ps = m._params()
+        with torch.enable_grad():
+            xi = x.detach().requires_grad_(ctx.needs_input_grad[0])
+            y, ld = m._reverse_formulas(xi)
+            wanted = [xi] if ctx.needs_input_grad[0] else []
+            wanted += [p for p, need in zip(ps, ctx.needs_input_grad[3:]) if need]
+            outs, gouts = [y], [dy]
+            if dlogdet is not None:
+                outs.append(ld)
+                gouts.append(dlogdet)
+            grads = list(torch.autograd.grad(outs, wanted, gouts, allow_unused=True))
+        dx = grads.pop(0) if ctx.needs_input_grad[0] else None
+        dps = [grads.pop(0) if need else None for need in ctx.needs_input_grad[3:]]
+        return (dx, None, None, *dps)
+
+
 class GaussianPrior(nn.Module):
     """standard normal over `size`; closed form, device follows the input / `device`"""
 
@@ -367,6 +430,13 @@ class SplitPrior(FlowLayer):
             x2 = torch.randn_like(input)
         return self.transform.reverse(torch.cat([input, x2], dim=1), context)
 
+    def reverse_and_logdet(self, input, x2=None):
+        """(reverse(input, x2), minus the term the forward adds: the coupling's reverse log-det - log N(x2))"""
+        if x2 is None:
+            x2 = torch.randn_like(input)
+        x, ld = self.transform.reverse_and_logdet(torch.cat([input, x2], dim=1))
+        return x, ld - self.base.log_prob(x2)
+
     def logdet(self, input, context=None):
         return self.forward(input, context)[2]
 
@@ -408,6 +478,26 @@ class Preprocess(nn.Module):
             x = layer.reverse(x)
         return x
 
+    def reverse_and_logdet(self, x):
+        """(reverse(x, quantize=False), log|det| of that map): the Normalization and LogitTransform terms of the
+        forward, negated, each at the forward's input; Dequantization adds 0"""
+        return _reverse_and_logdet(self.layers[1:], x)
+
+
+def _reverse_and_logdet(layers, x):
+    """x through the layers' reverse, last layer first, and the sum of their reverse log-determinants.  Each term is
+    minus what the layer's forward adds, evaluated where the forward evaluates it (the forward's input = the reverse's
+    output): the layer's own `reverse_and_logdet` where it has one, -layer.logdet(output) otherwise."""
+    logdet = 0
+    for layer in reversed(layers):
+        if hasattr(layer, "reverse_and_logdet"):
+            x, ld = layer.reverse_and_logdet(x)
+        else:
+            x = layer.reverse(x)
+            ld = -layer.logdet(x)
+        logdet = logdet + ld
+    return x, logdet
+
 
 class _Chain(nn.Module):
     def _fwd(self, seq, x):
@@ -442,8 +532,13 @@ class GlowStep(_Chain):
 
     def reverse(self, x):
         if self.fused and x.is_cuda:
-            return _fused_glow_reverse(self, x)
+            return _fused_glow_reverse(self, x, False)[0]
         return self._rev(self.glow_step, x)
+
+    def reverse_and_logdet(self, x):
+        if self.fused and x.is_cuda:
+            return _fused_glow_reverse(self, x, True)
+        return _reverse_and_logdet(self.glow_step, x)
 
 
 class _Affine1x1Fn(torch.autograd.Function):
@@ -490,9 +585,11 @@ class _InverseFn(torch.autograd.Function):
 
     @staticmethod
     def backward(ctx, g):
+        # -W^-T g W^-T as two finc_affine1x1_f32 products (a C x C matrix is one image of C channels, C pixels)
         (Winv,) = ctx.saved_tensors
-        WinvT = Winv.t()
-        return -(WinvT @ g @ WinvT)
+        C = Winv.shape[0]
+        P = _native.affine1x1(g.contiguous().view(1, C, C), Winv.t().contiguous())[0]     # W^-T g
+        return -_native.affine1x1(P.t().contiguous().view(1, C, C), Winv)[0].t()          # (W^-1 P^T)^T = P W^-T
 
 
 class _SlogdetFn(torch.autograd.Function):
@@ -564,25 +661,39 @@ def _fused_glow_forward(self, x):
     ld_w = conv.__dict__.pop("_ld_batched", None)     # set by FastFlow.forward: one batched LU per level
     if ld_w is None:
         ld_w = torch.slogdet(conv.W)[1]
-    ld_pix = ld_w if act is None else ld_w - act.log_scale.sum()
+    ld_pix = _affine_ld_pix(act, ld_w)
     y, ld = gs.coupling(y)
     return y, ld + (H * W) * ld_pix
 
 
-def _fused_glow_reverse(self, z):
+def _affine_ld_pix(act, ld_w):
+    """log|det| per pixel of [ActNorm +] Conv1x1 from ld_w = log|det W|"""
+    return ld_w if act is None else ld_w - act.log_scale.sum()
+
+
+def _fused_glow_reverse(self, z, want_logdet):
+    """(x, its reverse log-det: the coupling's and minus H*W*ld_pix, the affine term the forward adds; None unless
+    `want_logdet`)"""
     gs = self.glow_step
     act = getattr(gs, "actnorm", None)
     assert act is None or act.is_initialized()
-    x = gs.coupling.reverse(z)
+    x, ld = gs.coupling._reverse(z, want_logdet)
+    HW = z.shape[2] * z.shape[3]
     act_ps = [act.translation, act.log_scale] if act is not None else []
     if reverse_records(x, gs.conv1x1.W, *act_ps):
         # differentiable: A^-1 = exp(log_s)[:, None] W^-1 and the bias t, computed as _glue_constants does (same bits)
         W = gs.conv1x1.W
-        Winv = _InverseFn.apply(W) if W.is_cuda and W.shape[0] <= 128 else torch.inverse(W)
+        small = W.is_cuda and W.shape[0] <= 128
+        Winv = _InverseFn.apply(W) if small else torch.inverse(W)
         Ainv = Winv if act is None else torch.exp(act.log_scale).unsqueeze(1) * Winv
-        return _Affine1x1Fn.apply(x, Ainv, None if act is None else act.translation)
-    _, _, _, Ainv, binv = _glue_constants(self)
-    return _native.affine1x1(x.contiguous(), Ainv, binv)
+        y = _Affine1x1Fn.apply(x, Ainv, None if act is None else act.translation)
+        if want_logdet:
+            ld_w = _SlogdetFn.apply(W.unsqueeze(0))[0] if small else torch.slogdet(W)[1]
+            ld = ld - HW * _affine_ld_pix(act, ld_w)
+        return y, ld
+    _, _, ld_pix, Ainv, binv = _glue_constants(self)
+    y = _native.affine1x1(x.contiguous(), Ainv, binv)
+    return y, (ld - HW * ld_pix if want_logdet else None)
 
 
 class FastFlowStep(_Chain):
@@ -623,6 +734,9 @@ class FastFlowStep(_Chain):
     def reverse(self, x):
         return self._rev(self.fastflow_step, x)
 
+    def reverse_and_logdet(self, x):
+        return _reverse_and_logdet(self.fastflow_step, x)
+
 
 class FastFlowLevel(nn.Module):
     def __init__(self, size, block_size=16, actnorm=False, kernel_size=(3, 3), width=512, mask_in_backward=True):
@@ -647,6 +761,12 @@ class FastFlowLevel(nn.Module):
         for layer in reversed(self.fastflow_level):
             x = layer.reverse(x, z) if isinstance(layer, SplitPrior) else layer.reverse(x)
         return x
+
+    def reverse_and_logdet(self, x, z=None):
+        split = self.fastflow_level[-1]
+        x, ld = split.reverse_and_logdet(x, z)
+        x, ld_rest = _reverse_and_logdet(self.fastflow_level[:-1], x)
+        return x, ld + ld_rest
 
 
 class FastFlow(nn.Module):
@@ -713,6 +833,21 @@ class FastFlow(nn.Module):
         for i, level in enumerate(reversed(self.fastflow_levels)):
             x = level.reverse(x) if len(zs) == 1 else level.reverse(x, zs[-i - 2])
         return self.preprocess.reverse(x, quantize=quantize)
+
+    def sample_with_log_prob(self, n_samples=1, zs=None):
+        """(x, log_q[B]): x = reverse(n_samples, zs, quantize=False), the continuous image, and log_q its log-density
+        under the model in nats, log N(every latent, the split-prior ones drawn inside included) - log|det dx/dz|.
+        This is model.log_prob(x) with zero dequantisation noise, without a second pass.  Differentiable in `zs` and
+        the parameters wherever reverse() records a graph (reverse-KL: E_q[log q(x) - log p*(x)])."""
+        if zs is None:
+            zs = [self.base_distribution.sample(n_samples)[0]]
+        z, logdet = _reverse_and_logdet(self.fastflow_step, zs[-1])
+        x = self.squeeze.reverse(z)
+        for i, level in enumerate(reversed(self.fastflow_levels)):
+            x, ld = level.reverse_and_logdet(x) if len(zs) == 1 else level.reverse_and_logdet(x, zs[-i - 2])
+            logdet = logdet + ld
+        x, ld = self.preprocess.reverse_and_logdet(x)
+        return x, self.base_distribution.log_prob(zs[-1]) - (logdet + ld)
 
     def log_prob(self, x, bits_per_pixel=False):
         """bits_per_pixel: per IMAGE dimension (x[0].numel()).  The reference divides by `zs[0].numel()`, a

@@ -59,6 +59,7 @@ extern "C" {
 #define FINC_FLAG_TF32_1PASS 1024u /* tensor-core entry points: single-pass TF32 products (PyTorch's default conv precision, ~5e-4) instead of the fp32-accurate 3xTF32 split */
 #define FINC_FLAG_CHAIN_TRANSPOSE 2048u /* finc_chain_f32: backward-data chain (transposed weights, opposite corner) */
 #define FINC_FLAG_NEGATE 4096u /* backward_weight (and _batched): dw = -result (dw += -result with FINC_FLAG_ACCUMULATE); masked entries stay +0 */
+#define FINC_FLAG_COUPLING_REVERSE 8192u /* finc_coupling_backward_f32: the backward of the reverse direction (finc_coupling_apply_f32 with reverse = 1) */
 
 /* error codes (negative); positive return values are cudaError_t */
 #define FINC_OK 0
@@ -271,7 +272,10 @@ int finc_tc_wgrad_f32(const float* P, const float* Q, float* dW, void* workspace
 /* Affine coupling layer (fastflow/layers/coupling.py:44-105) in four launches:
  *   h = Conv2dZero(relu(conv1x1(relu(conv3x3(x[:, :C/2])))));  log_s = 2 tanh(h[:, ::2] / 2);  t = h[:, 1::2]
  *   forward:  y = cat(x1, x2 * exp(log_s) + t),   logdet[n] (+)= sum log_s        (Coupling.forward)
- *   reverse:  y = cat(x1, (x2 - t) * exp(-log_s))                               (Coupling.reverse)
+ *   reverse:  y = cat(x1, (x2 - t) * exp(-log_s)), logdet[n] (+)= -sum log_s      (Coupling.reverse)
+ * `logdet` (nullable, [B]) is log|det dy/dx| of the direction that runs: with reverse = 1 it is minus the forward's
+ * log-det at the reconstructed input (the log-density term of a sample); one more launch when given.
+ * FINC_FLAG_LOGDET_ACCUMULATE adds into it in both directions.
  * x, y: NCHW [B, C, H, W] (y == x allowed); the hidden activations stay channels-last in `workspace`.
  * `prepared` = finc_coupling_prepare_f32(net.0.weight [width,C/2,3,3], net.0.bias, net.2.weight
  * [width,width,1,1], net.2.bias, net.4.weight [C,width,3,3], net.4.bias, net.4.logs, logscale_factor).
@@ -286,13 +290,16 @@ int finc_coupling_apply_f32(const float* x, float* y, float* logdet, const void*
                             size_t workspace_bytes, int B, int C, int H, int W, int width, int reverse,
                             unsigned flags, void* stream);
 
-/* Backward of finc_coupling_apply_f32 (forward direction): given dy = dL/dy and dlogdet = dL/dlogdet [B] (may be
- * NULL) it produces dx and the gradients of the seven parameters (same shapes as the parameters).
- * `forward_workspace` is the workspace the forward call filled (it holds the hidden activations) and `prepared`
- * a blob made with with_backward = 1 (it carries the transposed weights).  Eleven GEMM-class launches on the
+/* Backward of finc_coupling_apply_f32: given dy = dL/dy and dlogdet = dL/dlogdet [B] (may be NULL) it produces dx and
+ * the gradients of the seven parameters (same shapes as the parameters).
+ * `forward_workspace` is the workspace the apply call filled (it holds the hidden activations), `x` that call's input
+ * and `prepared` a blob made with with_backward = 1 (it carries the transposed weights).  Without flags this is the
+ * backward of the forward direction (reverse = 0); with FINC_FLAG_COUPLING_REVERSE it is the backward of the reverse
+ * direction (reverse = 1), `dlogdet` then being the gradient of the reverse log-det -sum log_s.  The network
+ * h = net(x1) is the same in both directions, so only the pointwise step differs.  Eleven GEMM-class launches on the
  * tensor cores (three weight-gradient GEMMs over the pixels, three backward-data GEMMs) plus small
  * deterministic reductions; no floating-point atomics.  width % 128 == 0.  Replaces the autograd graph of
- * Coupling.forward (fastflow/layers/coupling.py:85-90; cuDNN dgrad / wgrad). */
+ * Coupling.forward / Coupling.reverse (fastflow/layers/coupling.py:85-99; cuDNN dgrad / wgrad). */
 size_t finc_coupling_backward_workspace_bytes(int B, int C, int H, int W, int width);
 int finc_coupling_backward_f32(const float* x, const float* dy, const float* dlogdet, const void* prepared,
                                const void* forward_workspace, void* scratch, size_t scratch_bytes, float* dx,
