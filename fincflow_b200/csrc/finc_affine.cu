@@ -528,11 +528,14 @@ __global__ void slogdet_inverse_kernel(const float* __restrict__ W, float* __res
 int launch_slogdet_inverse(const float* W, float* logabsdet, float* Winv, int n, int C, cudaStream_t st) {
     if (n == 0) return 0;
     const size_t smem = ((size_t)C * (2 * C + 1) + C) * sizeof(float);
-    static bool configured = false;
-    if (smem > 48 * 1024 && !configured) {
+    // the opt-in limit is a function attribute of the device's context: raise it once per device, not per process
+    static bool configured[64] = {};
+    int dev = 0;
+    if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) dev = -1;
+    if (smem > 48 * 1024 && (dev < 0 || !configured[dev])) {
         cudaError_t err = cudaFuncSetAttribute(slogdet_inverse_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
         if (err != cudaSuccess) return (int)err;
-        configured = true;
+        if (dev >= 0) configured[dev] = true;
     }
     slogdet_inverse_kernel<<<n, 128, smem, st>>>(W, logabsdet, Winv, C);
     return (int)cudaGetLastError();

@@ -413,6 +413,7 @@ struct Plan {
 // more Z = shorter partial vectors but every slice re-reads the tiles.  A small cost model
 // (microseconds, calibrated with tools/kernel_timeline.py) picks the cheapest combination.
 bool make_plan(const Shape& s, Plan* p, int sm_div = 1) {
+    if (s.B < 1) return false;  // no chunks to spread: the per-CTA chunk count would divide by zero
     if (!(s.kH == s.kW && (s.kH == 3 || s.kH == 5))) return false;
     int WT;
     if (s.W % 4 == 0) WT = 4;

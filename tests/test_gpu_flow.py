@@ -23,7 +23,9 @@ def _ref_space_to_depth(x):  # the formula of layers/squeeze.py:5-13
     return x.view(xs[0], xs[1] * 4, xs[2] // 2, xs[3] // 2)
 
 
-@pytest.mark.parametrize("shape", [(3, 3, 32, 32), (5, 1, 28, 28), (2, 12, 16, 16), (1, 6, 2, 2), (256, 3, 32, 32)])
+@pytest.mark.parametrize("shape", [(3, 3, 32, 32), (5, 1, 28, 28), (2, 12, 16, 16), (1, 6, 2, 2), (256, 3, 32, 32),
+                                   (64, 12, 64, 64),            # 1.6M float2 items: more than the grid's 148 * 32 * 256
+                                   (3, 5, 30, 30), (2, 3, 6, 10)])   # odd H/2 and W/2
 def test_squeeze_kernels_bit_exact(shape):
     from fincflow_b200 import _native
 

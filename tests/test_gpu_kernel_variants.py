@@ -56,19 +56,42 @@ UNREACHABLE = {
 
 
 def _arg(v):
-    v = v.strip()
-    return {"true": 1, "false": 0}[v] if v in ("true", "false") else int(v)
+    v = " ".join(v.split())
+    if v in ("true", "false"):
+        return int(v == "true")
+    return int(v) if re.fullmatch(r"-?\d+", v) else v   # a type argument stays a string
+
+
+def _template_args(s):
+    """the arguments of the template argument list `s` starts with ("<...>", nesting allowed) and its length"""
+    depth, args, start = 0, [], 1
+    for i, ch in enumerate(s):
+        if ch == "<":
+            depth += 1
+        elif ch == ">":
+            depth -= 1
+            if depth == 0:
+                args.append(s[start:i])
+                return tuple(_arg(a) for a in args), i + 1
+        elif ch == "," and depth == 1:
+            args.append(s[start:i])
+            start = i + 1
+    raise ValueError(f"unbalanced template arguments in {s!r}")
 
 
 def kernels_in(names, families=FAMILIES):
-    """{(family, template arguments)} of the kernel families in `families` (name -> qualified template name, by
-    default the five FInC families) among kernel names (bools as 0 / 1)"""
-    pattern = re.compile("(" + "|".join(re.escape(p) for p in families.values()) + r")<([^<>]*)>")
+    """{(family, template arguments)} of the kernel families in `families` (name -> qualified kernel name, by
+    default the five FInC families) among kernel names.  Bools read as 0 / 1 and type arguments as strings; a
+    kernel that is not a template (its name followed by its parameter list, or an unmangled extern "C" name alone)
+    has the arguments ()."""
+    pattern = re.compile(r"(?<![\w:])(" + "|".join(re.escape(p) for p in families.values()) + r")(?=[<(]|$)")
     family_of = {p: f for f, p in families.items()}
     found = set()
     for name in names:
-        for prefix, args in pattern.findall(name):
-            found.add((family_of[prefix], tuple(_arg(a) for a in args.split(","))))
+        for m in pattern.finditer(name):
+            rest = name[m.end():]
+            args = _template_args(rest)[0] if rest.startswith("<") else ()
+            found.add((family_of[m.group(1)], args))
     return found
 
 

@@ -242,18 +242,18 @@ def test_fused_adam_matches_torch():
     from fincflow_b200 import _native
 
     torch.manual_seed(0)
-    n = 10007
-    p0 = torch.randn(n, device="cuda")
-    ref = p0.clone().requires_grad_(True)
-    opt = torch.optim.Adam([ref], lr=1e-3)
-    p, m, v, step = p0.clone(), torch.zeros(n, device="cuda"), torch.zeros(n, device="cuda"), torch.zeros(1, device="cuda")
-    for it in range(5):
-        g = torch.randn(n, device="cuda")
-        ref.grad = g.clone()
-        opt.step()
-        _native.adam_step_(p, g, m, v, step, lr=1e-3)
-    assert step.item() == 5.0
-    assert torch.allclose(p, ref.detach(), rtol=1e-5, atol=1e-6)
+    for n in (10007, 1000003):   # 1000003 > SMs * 8 * 256: the grid-stride loop runs more than one pass
+        p0 = torch.randn(n, device="cuda")
+        ref = p0.clone().requires_grad_(True)
+        opt = torch.optim.Adam([ref], lr=1e-3)
+        p, m, v, step = p0.clone(), torch.zeros(n, device="cuda"), torch.zeros(n, device="cuda"), torch.zeros(1, device="cuda")
+        for it in range(5):
+            g = torch.randn(n, device="cuda")
+            ref.grad = g.clone()
+            opt.step()
+            _native.adam_step_(p, g, m, v, step, lr=1e-3)
+        assert step.item() == 5.0
+        assert torch.allclose(p, ref.detach(), rtol=1e-5, atol=1e-6)
 
 
 def _run_steps(levels, B, n_steps, **kw):

@@ -46,6 +46,7 @@ def test_abi_version_and_error_strings(lib_path):
     assert lib.finc_forward_f32(None, None, None, None, 1, 4, 3, 8, 8, 3, 3, 0xE4, 0, None) == -1
     assert lib.finc_inverse_f32(None, None, None, 1, 17, 3, 8, 8, 3, 3, 0, 0, None) == -1  # G > 16
     assert lib.finc_backward_weight_workspace_bytes(256, 4, 3, 16, 16, 3, 3) >= 4096
+    assert lib.finc_backward_weight_workspace_bytes(0, 4, 3, 16, 16, 3, 3) >= 4096   # B = 0: no plan, no division
     # tensor-core entry points: sizes are host arithmetic, bad arguments are rejected before any CUDA call
     assert lib.finc_coupling_prepared_bytes(12, 512, 0) > 4 * (2 * 512 * 64 + 2 * 512 * 512 + 2 * 9 * 16 * 512)
     assert lib.finc_coupling_prepared_bytes(12, 512, 1) > lib.finc_coupling_prepared_bytes(12, 512, 0)
@@ -58,6 +59,19 @@ def test_abi_version_and_error_strings(lib_path):
     assert lib.finc_coupling_apply_f32(None, None, None, None, None, 0, 1, 12, 8, 8, 512, 0, 0, None) == -1
     assert lib.finc_tc_conv_nhwc_f32(None, None, None, None, None, 1, 8, 8, 32, 32, 9, 0, 0, None) == -1
     assert lib.finc_tc_conv_weights_bytes(512, 6, 9, 1) == 2 * 512 * 64 * 4
+    # glue entry points: the edges they refuse, before any CUDA call
+    f, nil = ctypes.c_float, ctypes.c_void_p(16)   # a non-null, 16-byte aligned pointer that is never dereferenced
+    assert lib.finc_affine1x1_f32(nil, nil, None, ctypes.c_void_p(32), 1, 4097, 16, None) == -1        # C > 4096
+    assert lib.finc_affine1x1_backward_weight_workspace_bytes(1, 4097, 16) == 0
+    assert lib.finc_slogdet_inverse_f32(nil, nil, nil, 3, 129, None) == -1                           # C > 128
+    assert lib.finc_preprocess_f32(nil, None, nil, None, 1, 10, f(0.5), 0, None) == -1               # alpha >= 0.5
+    assert lib.finc_squeeze_f32(nil, ctypes.c_void_p(64), 1, 3, 7, 8, None) == -1                    # odd H
+    assert lib.finc_squeeze_f32(nil, ctypes.c_void_p(64), 1, 3, 8, 7, None) == -1                    # odd W
+    assert lib.finc_squeeze_f32(ctypes.c_void_p(20), ctypes.c_void_p(64), 1, 3, 8, 8, None) == -1    # x 4-byte aligned
+    # a workspace one float too small for the tiled affine weight gradient: FINC_E_WORKSPACE, nothing launched
+    need = lib.finc_affine1x1_backward_weight_workspace_bytes(2, 16, 64)
+    assert need > 64
+    assert lib.finc_affine1x1_backward_weight_f32(nil, nil, nil, None, nil, need - 4, 2, 16, 64, None) == -2
 
 
 def test_sass_is_sm100a_with_bulk_tma(lib_path):
@@ -123,3 +137,34 @@ def test_layer_api_matches_reference_surface():
     assert unit.conv_br.conv.weight.shape == (3, 3, 3, 3) and unit.conv_br.order == "BR"
     with pytest.raises(AssertionError):
         FastFlowUnit(6, 6, (3, 3))
+
+
+def test_every_kernel_belongs_to_exactly_one_census(lib_path):
+    """every kernel entry of the library (template instantiations from the symbol table, the others from their
+    __device_stub__ symbols) belongs to exactly one of the three census family maps: FInC
+    (test_gpu_kernel_variants.py), tensor-core (test_gpu_tc_variants.py) and glue (test_gpu_glue_variants.py), so a
+    new kernel anywhere has to be claimed by a census.  Cross-checked against cuobjdump's function count."""
+    import shutil
+    import subprocess
+
+    if not (shutil.which("nm") and shutil.which("c++filt")):
+        pytest.skip("nm / c++filt not available")
+    from test_gpu_glue_variants import GLUE_FAMILIES, kernel_entries
+    from test_gpu_kernel_variants import FAMILIES
+    from test_gpu_tc_variants import TC_FAMILIES
+
+    entries = kernel_entries(lib_path)
+    maps = {"finc": FAMILIES, "tc": TC_FAMILIES, "glue": GLUE_FAMILIES}
+    owners = {}
+    for name, args in entries:
+        owners[(name, args)] = [m for m, fams in maps.items() if name in fams.values()]
+    unclaimed = sorted(e for e, o in owners.items() if not o)
+    assert not unclaimed, f"kernels no census claims: {unclaimed}"
+    assert all(len(o) == 1 for o in owners.values())
+    counts = {m: sum(1 for o in owners.values() if o == [m]) for m in maps}
+    print(f"\n[library census] {len(entries)} kernel entries: {counts}")
+    cuobjdump = shutil.which("cuobjdump") or "/usr/local/cuda/bin/cuobjdump"
+    if os.path.exists(cuobjdump):
+        out = subprocess.run([cuobjdump, "-res-usage", lib_path], capture_output=True, text=True).stdout
+        functions = set(re.findall(r"^\s*Function (\S+?):", out, flags=re.M))
+        assert len(functions) == len(entries), (len(functions), len(entries))
