@@ -264,24 +264,28 @@ class Coupling(FlowLayer):
         log_s = 2.0 * torch.tanh(h[:, ::2] / 2.0)
         return x1, x2, log_s, h[:, 1::2]
 
+    def _formulas(self, x, reverse):
+        """(y, the direction's log-det [B]): forward y2 = x2 exp(log_s) + t, sum log_s; reverse
+        y2 = (x2 - t) exp(-log_s), -sum log_s"""
+        x1, x2, log_s, t = self._st(x)
+        ld = log_s.flatten(start_dim=1).sum(-1)
+        if reverse:
+            return torch.cat([x1, (x2 - t) * torch.exp(-log_s)], dim=1), -ld
+        return torch.cat([x1, x2 * torch.exp(log_s) + t], dim=1), ld
+
     def forward(self, input, context=None):
         if self._use_tc(input):
-            return _CouplingFn.apply(input, self, *self._params())
-        x1, x2, log_s, t = self._st(input)
-        return torch.cat([x1, x2 * torch.exp(log_s) + t], dim=1), log_s.flatten(start_dim=1).sum(-1)
-
-    def _reverse_formulas(self, x):
-        x1, x2, log_s, t = self._st(x)
-        return torch.cat([x1, (x2 - t) * torch.exp(-log_s)], dim=1), -log_s.flatten(start_dim=1).sum(-1)
+            return _CouplingFn.apply(input, self, False, True, *self._params())
+        return self._formulas(input, False)
 
     def _reverse(self, input, want_logdet):
         if self._use_tc(input):
             # a graph exactly when the formulas below would record one
             if torch.is_grad_enabled() and (input.requires_grad or any(p.requires_grad for p in self._params())):
-                return _CouplingReverseFn.apply(input, self, want_logdet, *self._params())
+                return _CouplingFn.apply(input, self, True, want_logdet, *self._params())
             return _native.coupling_apply(input, self.prepared(), self.width, reverse=True, want_logdet=want_logdet,
                                           flags=self._flags())
-        y, ld = self._reverse_formulas(input)
+        y, ld = self._formulas(input, True)
         return y, (ld if want_logdet else None)
 
     def reverse(self, input, context=None):
@@ -296,14 +300,15 @@ class Coupling(FlowLayer):
 
 
 class _CouplingFn(torch.autograd.Function):
-    """Coupling.forward and its backward on the tensor-core kernels (finc_coupling_apply_f32 /
-    finc_coupling_backward_f32).  The forward keeps its workspace (the channels-last hidden activations)
-    for the backward.  Widths the backward kernels do not cover (width % 128 != 0) recompute through the
-    PyTorch formulas instead."""
+    """Coupling.forward, or with `reverse` its reverse (and the reverse's log-det -sum log_s when `want_logdet`; None
+    otherwise), with the backward on the tensor-core kernels: finc_coupling_apply_f32, then one
+    finc_coupling_backward_f32 on the kept workspace (the channels-last hidden activations), with
+    FINC_FLAG_COUPLING_REVERSE for the reverse.  Widths the backward kernels do not cover (width % 128 != 0)
+    recompute through the PyTorch formulas instead."""
 
     @staticmethod
-    def forward(ctx, x, module, *params):
-        ctx.module = module
+    def forward(ctx, x, module, reverse, want_logdet, *params):
+        ctx.module, ctx.reverse = module, reverse
         B, C, H, W = x.shape
         train = any(ctx.needs_input_grad)
         ctx.native = train and _native.coupling_prepared_bytes(C, module.width, True) > 0
@@ -311,51 +316,7 @@ class _CouplingFn(torch.autograd.Function):
         if ctx.native:
             ws = torch.empty(_native.coupling_workspace_bytes(B, C, H, W, module.width), dtype=torch.uint8, device=x.device)
         blob = module.prepared(with_backward=ctx.native, training=train)
-        y, logdet = _native.coupling_apply(x, blob, module.width, flags=module._flags(), workspace=ws)
-        ctx.save_for_backward(x)
-        ctx.ws, ctx.blob = ws, blob
-        return y, logdet
-
-    @staticmethod
-    def backward(ctx, dy, dlogdet):
-        (x,) = ctx.saved_tensors
-        m = ctx.module
-        if ctx.native:
-            if dy is None:
-                dy = torch.zeros_like(x)
-            grads = _native.coupling_backward(x, dy.contiguous(), dlogdet, ctx.blob, ctx.ws, m.width, flags=m._flags())
-            ctx.ws = None
-            return (grads[0], None, *grads[1:])
-        ps = m._params()
-        with torch.enable_grad():
-            xi = x.detach().requires_grad_(ctx.needs_input_grad[0])
-            x1, x2, log_s, t = m._st(xi)
-            y = torch.cat([x1, x2 * torch.exp(log_s) + t], dim=1)
-            ld = log_s.flatten(start_dim=1).sum(-1)
-            wanted = [xi] if ctx.needs_input_grad[0] else []
-            wanted += [p for p, need in zip(ps, ctx.needs_input_grad[2:]) if need]
-            grads = list(torch.autograd.grad([y, ld], wanted, [dy, dlogdet], allow_unused=True))
-        dx = grads.pop(0) if ctx.needs_input_grad[0] else None
-        dps = [grads.pop(0) if need else None for need in ctx.needs_input_grad[2:]]
-        return (dx, None, *dps)
-
-
-class _CouplingReverseFn(torch.autograd.Function):
-    """Coupling.reverse (and its log-det -sum log_s when `want_logdet`) with its backward on the tensor-core kernels:
-    finc_coupling_apply_f32(reverse = 1), then one finc_coupling_backward_f32 with FINC_FLAG_COUPLING_REVERSE on the
-    kept workspace.  Widths the backward kernels do not cover (width % 128 != 0) recompute through the PyTorch
-    formulas instead, as _CouplingFn does."""
-
-    @staticmethod
-    def forward(ctx, x, module, want_logdet, *params):
-        ctx.module = module
-        B, C, H, W = x.shape
-        ctx.native = _native.coupling_prepared_bytes(C, module.width, True) > 0
-        ws = None
-        if ctx.native:
-            ws = torch.empty(_native.coupling_workspace_bytes(B, C, H, W, module.width), dtype=torch.uint8, device=x.device)
-        blob = module.prepared(with_backward=ctx.native, training=True)
-        y, logdet = _native.coupling_apply(x, blob, module.width, reverse=True, want_logdet=want_logdet,
+        y, logdet = _native.coupling_apply(x, blob, module.width, reverse=reverse, want_logdet=want_logdet,
                                            flags=module._flags(), workspace=ws)
         ctx.save_for_backward(x)
         ctx.ws, ctx.blob = ws, blob
@@ -368,24 +329,24 @@ class _CouplingReverseFn(torch.autograd.Function):
         if ctx.native:
             if dy is None:
                 dy = torch.zeros_like(x)
-            grads = _native.coupling_backward(x, dy.contiguous(), dlogdet, ctx.blob, ctx.ws, m.width,
-                                              flags=m._flags() | _native.FLAG_COUPLING_REVERSE)
+            flags = m._flags() | (_native.FLAG_COUPLING_REVERSE if ctx.reverse else 0)
+            grads = _native.coupling_backward(x, dy.contiguous(), dlogdet, ctx.blob, ctx.ws, m.width, flags=flags)
             ctx.ws = None
-            return (grads[0], None, None, *grads[1:])
+            return (grads[0], None, None, None, *grads[1:])
         ps = m._params()
         with torch.enable_grad():
             xi = x.detach().requires_grad_(ctx.needs_input_grad[0])
-            y, ld = m._reverse_formulas(xi)
+            y, ld = m._formulas(xi, ctx.reverse)
             wanted = [xi] if ctx.needs_input_grad[0] else []
-            wanted += [p for p, need in zip(ps, ctx.needs_input_grad[3:]) if need]
+            wanted += [p for p, need in zip(ps, ctx.needs_input_grad[4:]) if need]
             outs, gouts = [y], [dy]
-            if dlogdet is not None:
+            if dlogdet is not None:    # None: a reverse without its log-det
                 outs.append(ld)
                 gouts.append(dlogdet)
             grads = list(torch.autograd.grad(outs, wanted, gouts, allow_unused=True))
         dx = grads.pop(0) if ctx.needs_input_grad[0] else None
-        dps = [grads.pop(0) if need else None for need in ctx.needs_input_grad[3:]]
-        return (dx, None, None, *dps)
+        dps = [grads.pop(0) if need else None for need in ctx.needs_input_grad[4:]]
+        return (dx, None, None, None, *dps)
 
 
 class GaussianPrior(nn.Module):
@@ -425,17 +386,18 @@ class SplitPrior(FlowLayer):
         x1, x2 = x[:, :self.n_channels // 2], x[:, self.n_channels // 2:]
         return x1, x2, self.base.log_prob(x2) + ldj
 
-    def reverse(self, input, x2=None, context=None):
+    def _reverse(self, input, x2, want_logdet):
+        """(x, minus the term the forward adds: the coupling's reverse log-det - log N(x2); None unless `want_logdet`)"""
         if x2 is None:
             x2 = torch.randn_like(input)
-        return self.transform.reverse(torch.cat([input, x2], dim=1), context)
+        x, ld = self.transform._reverse(torch.cat([input, x2], dim=1), want_logdet)
+        return x, (ld - self.base.log_prob(x2) if want_logdet else None)
+
+    def reverse(self, input, x2=None, context=None):
+        return self._reverse(input, x2, False)[0]
 
     def reverse_and_logdet(self, input, x2=None):
-        """(reverse(input, x2), minus the term the forward adds: the coupling's reverse log-det - log N(x2))"""
-        if x2 is None:
-            x2 = torch.randn_like(input)
-        x, ld = self.transform.reverse_and_logdet(torch.cat([input, x2], dim=1))
-        return x, ld - self.base.log_prob(x2)
+        return self._reverse(input, x2, True)
 
     def logdet(self, input, context=None):
         return self.forward(input, context)[2]
@@ -463,57 +425,52 @@ class Preprocess(nn.Module):
             deq = self.layers[0]
             u = deq.fixed_noise.to(x.device) if deq.fixed_noise is not None else torch.rand_like(x)
             return _native.preprocess(x, u, self.alpha)
-        logdet = 0
-        for layer in self.layers:
-            x, ld = layer(x)
-            logdet = logdet + ld
-        return x, logdet
+        return _forward_layers(self.layers, x)
+
+    def _reverse(self, x, want_logdet, quantize=False):
+        """(reverse(x, quantize), log|det| of that map or None unless `want_logdet`).  The log-det is that of the
+        continuous image (quantize=False): the Normalization and LogitTransform terms of the forward, negated, each at
+        the forward's input; Dequantization adds 0."""
+        if quantize and self.fused and x.is_cuda and x.dtype == torch.float32 and not torch.is_grad_enabled():
+            return _native.preprocess(x, None, self.alpha, reverse=True)[0], None
+        return _reverse_layers(self.layers if quantize else self.layers[1:], x, want_logdet)
 
     def reverse(self, x, quantize=True):
         """`quantize=False` stops before Dequantization's floor and returns the continuous image in [0, 256), whose
         gradient reaches the latents and the parameters (the floored image has zero gradient everywhere)."""
-        if quantize and self.fused and x.is_cuda and x.dtype == torch.float32 and not torch.is_grad_enabled():
-            return _native.preprocess(x, None, self.alpha, reverse=True)[0]
-        for layer in reversed(self.layers if quantize else self.layers[1:]):
-            x = layer.reverse(x)
-        return x
+        return self._reverse(x, False, quantize)[0]
 
     def reverse_and_logdet(self, x):
-        """(reverse(x, quantize=False), log|det| of that map): the Normalization and LogitTransform terms of the
-        forward, negated, each at the forward's input; Dequantization adds 0"""
-        return _reverse_and_logdet(self.layers[1:], x)
+        return self._reverse(x, True)
 
 
-def _reverse_and_logdet(layers, x):
-    """x through the layers' reverse, last layer first, and the sum of their reverse log-determinants.  Each term is
-    minus what the layer's forward adds, evaluated where the forward evaluates it (the forward's input = the reverse's
-    output): the layer's own `reverse_and_logdet` where it has one, -layer.logdet(output) otherwise."""
+def _forward_layers(layers, x):
+    """x through the layers' forward, and the sum of their log-determinants"""
     logdet = 0
-    for layer in reversed(layers):
-        if hasattr(layer, "reverse_and_logdet"):
-            x, ld = layer.reverse_and_logdet(x)
-        else:
-            x = layer.reverse(x)
-            ld = -layer.logdet(x)
+    for layer in layers:
+        x, ld = layer(x)
         logdet = logdet + ld
     return x, logdet
 
 
-class _Chain(nn.Module):
-    def _fwd(self, seq, x):
-        logdet = 0
-        for layer in seq:
-            x, ld = layer(x)
-            logdet = logdet + ld
-        return x, logdet
-
-    def _rev(self, seq, x):
-        for layer in reversed(seq):
+def _reverse_layers(layers, x, want_logdet):
+    """x through the layers' reverse, last layer first, and (None unless `want_logdet`) the sum of their reverse
+    log-determinants.  Each term is minus what the layer's forward adds, evaluated where the forward evaluates it (the
+    forward's input = the reverse's output): the layer's own `_reverse` where it has one, -layer.logdet(output)
+    otherwise.  Without `want_logdet` no layer's logdet runs: some launch kernels or allocate."""
+    logdet = 0 if want_logdet else None
+    for layer in reversed(layers):
+        if hasattr(layer, "_reverse"):
+            x, ld = layer._reverse(x, want_logdet)
+        else:
             x = layer.reverse(x)
-        return x
+            ld = -layer.logdet(x) if want_logdet else None
+        if want_logdet:
+            logdet = logdet + ld
+    return x, logdet
 
 
-class GlowStep(_Chain):
+class GlowStep(nn.Module):
     def __init__(self, size, actnorm=False, width=512):
         super().__init__()
         d = OrderedDict()
@@ -528,17 +485,18 @@ class GlowStep(_Chain):
     def forward(self, x):
         if self.fused and x.is_cuda:
             return _fused_glow_forward(self, x)
-        return self._fwd(self.glow_step, x)
+        return _forward_layers(self.glow_step, x)
+
+    def _reverse(self, x, want_logdet):
+        if self.fused and x.is_cuda:
+            return _fused_glow_reverse(self, x, want_logdet)
+        return _reverse_layers(self.glow_step, x, want_logdet)
 
     def reverse(self, x):
-        if self.fused and x.is_cuda:
-            return _fused_glow_reverse(self, x, False)[0]
-        return self._rev(self.glow_step, x)
+        return self._reverse(x, False)[0]
 
     def reverse_and_logdet(self, x):
-        if self.fused and x.is_cuda:
-            return _fused_glow_reverse(self, x, True)
-        return _reverse_and_logdet(self.glow_step, x)
+        return self._reverse(x, True)
 
 
 class _Affine1x1Fn(torch.autograd.Function):
@@ -562,15 +520,6 @@ class _Affine1x1Fn(torch.autograd.Function):
         if ctx.needs_input_grad[1] or (ctx.has_bias and ctx.needs_input_grad[2]):
             dA, db = _native.affine1x1_backward_weight(dy, x, want_bias=ctx.has_bias)
         return dx, dA, db
-
-
-def affine_of(actnorm, conv1x1):
-    """(A, b) of ActNorm followed by Conv1x1: W ((x - t) * exp(-log_s)) = A x + b"""
-    W = conv1x1.W
-    if actnorm is None:
-        return W, None
-    A = W * torch.exp(-actnorm.log_scale).unsqueeze(0)
-    return A, -(A @ actnorm.translation)
 
 
 class _InverseFn(torch.autograd.Function):
@@ -607,6 +556,39 @@ class _SlogdetFn(torch.autograd.Function):
         return g.view(-1, 1, 1) * Winv.transpose(1, 2)
 
 
+def _native_slogdet(W):
+    """whether finc_slogdet_inverse_f32 takes the Conv1x1 weight(s) W: CUDA, at most 128 channels"""
+    return W.is_cuda and W.shape[-1] <= 128
+
+
+def _affine_map(act, conv, reverse, want_logdet=False, ld_w=None):
+    """(M, bias, ld_pix): one direction of [ActNorm +] Conv1x1 as the per-pixel affine map M x + bias, and the
+    log|det| per pixel of the forward map, ld_w - sum log_s where ld_w = log|det W|.
+      forward: M = A = W exp(-log_s)[None, :], bias = -A t; ld_pix from the caller's `ld_w`, None without one;
+      reverse: M = A^-1 = exp(log_s)[:, None] W^-1, bias = t; ld_pix when `want_logdet`, None otherwise.
+    bias is None without ActNorm.  Differentiable under grad, where W^-1 and log|det W| take one
+    finc_slogdet_inverse_f32 call each (_InverseFn, _SlogdetFn); under no_grad (_glue_constants) they come from one
+    call together, the same bits."""
+    W = M = conv.W
+    if reverse:
+        if not _native_slogdet(W):
+            M = torch.inverse(W)
+            ld_w = torch.slogdet(W)[1] if want_logdet else None
+        elif torch.is_grad_enabled():
+            M = _InverseFn.apply(W)
+            ld_w = _SlogdetFn.apply(W.unsqueeze(0))[0] if want_logdet else None
+        else:
+            ld, Winv = _native.slogdet_inverse(W.unsqueeze(0).contiguous())
+            M, ld_w = Winv[0], (ld[0] if want_logdet else None)
+    if act is None:
+        return M, None, ld_w
+    ld_pix = None if ld_w is None else ld_w - act.log_scale.sum()
+    if reverse:
+        return torch.exp(act.log_scale).unsqueeze(1) * M, act.translation, ld_pix
+    A = W * torch.exp(-act.log_scale).unsqueeze(0)
+    return A, -(A @ act.translation), ld_pix
+
+
 def _glue_constants(self):
     """(A, b, scalar logdet per pixel, A^-1, reverse bias) of [ActNorm +] Conv1x1, cached on the parameter
     versions.  Used under no_grad (evaluation / sampling): slogdet, inverse and the small products then run
@@ -618,21 +600,9 @@ def _glue_constants(self):
     key = tuple((p.data_ptr(), p._version) for p in ps)
     if getattr(self, "_glue_key", None) != key:
         with torch.no_grad():
-            W = conv.W.detach()
-            if W.is_cuda and W.shape[0] <= 128:
-                ld, Winv = _native.slogdet_inverse(W.unsqueeze(0).contiguous())
-                ld, Winv = ld[0], Winv[0]
-            else:
-                ld, Winv = torch.slogdet(W)[1], torch.inverse(W)
-            if act is None:
-                A, b, Ainv, binv = W, None, Winv, None
-            else:
-                A = W * torch.exp(-act.log_scale.detach()).unsqueeze(0)
-                b = -(A @ act.translation.detach())
-                ld = ld - act.log_scale.detach().sum()
-                Ainv = torch.exp(act.log_scale.detach()).unsqueeze(1) * Winv
-                binv = act.translation.detach().contiguous()
-            self._glue = (A.contiguous(), None if b is None else b.contiguous(), ld, Ainv.contiguous(), binv)
+            Ainv, binv, ld_pix = _affine_map(act, conv, True, want_logdet=True)
+            A, b, _ = _affine_map(act, conv, False)
+        self._glue = tuple(None if t is None else t.detach().contiguous() for t in (A, b, ld_pix, Ainv, binv))
         self._glue_key = key
     return self._glue
 
@@ -656,19 +626,13 @@ def _fused_glow_forward(self, x):
         return y, ld + (H * W) * ld_pix
     self._glue_key = None   # training forward: the cached evaluation constants may not be trusted afterwards
                             # (torch's fused Adam updates parameters without bumping their version counters)
-    A, b = affine_of(act, conv)
-    y = _Affine1x1Fn.apply(x, A, b)
     ld_w = conv.__dict__.pop("_ld_batched", None)     # set by FastFlow.forward: one batched LU per level
     if ld_w is None:
         ld_w = torch.slogdet(conv.W)[1]
-    ld_pix = _affine_ld_pix(act, ld_w)
+    A, b, ld_pix = _affine_map(act, conv, False, ld_w=ld_w)
+    y = _Affine1x1Fn.apply(x, A, b)
     y, ld = gs.coupling(y)
     return y, ld + (H * W) * ld_pix
-
-
-def _affine_ld_pix(act, ld_w):
-    """log|det| per pixel of [ActNorm +] Conv1x1 from ld_w = log|det W|"""
-    return ld_w if act is None else ld_w - act.log_scale.sum()
 
 
 def _fused_glow_reverse(self, z, want_logdet):
@@ -681,22 +645,15 @@ def _fused_glow_reverse(self, z, want_logdet):
     HW = z.shape[2] * z.shape[3]
     act_ps = [act.translation, act.log_scale] if act is not None else []
     if reverse_records(x, gs.conv1x1.W, *act_ps):
-        # differentiable: A^-1 = exp(log_s)[:, None] W^-1 and the bias t, computed as _glue_constants does (same bits)
-        W = gs.conv1x1.W
-        small = W.is_cuda and W.shape[0] <= 128
-        Winv = _InverseFn.apply(W) if small else torch.inverse(W)
-        Ainv = Winv if act is None else torch.exp(act.log_scale).unsqueeze(1) * Winv
-        y = _Affine1x1Fn.apply(x, Ainv, None if act is None else act.translation)
-        if want_logdet:
-            ld_w = _SlogdetFn.apply(W.unsqueeze(0))[0] if small else torch.slogdet(W)[1]
-            ld = ld - HW * _affine_ld_pix(act, ld_w)
-        return y, ld
-    _, _, ld_pix, Ainv, binv = _glue_constants(self)
-    y = _native.affine1x1(x.contiguous(), Ainv, binv)
+        Ainv, binv, ld_pix = _affine_map(act, gs.conv1x1, True, want_logdet)
+        y = _Affine1x1Fn.apply(x, Ainv, binv)
+    else:
+        _, _, ld_pix, Ainv, binv = _glue_constants(self)
+        y = _native.affine1x1(x.contiguous(), Ainv, binv)
     return y, (ld - HW * ld_pix if want_logdet else None)
 
 
-class FastFlowStep(_Chain):
+class FastFlowStep(nn.Module):
     def __init__(self, size, actnorm=False, kernel_size=(3, 3), width=512, mask_in_backward=True):
         super().__init__()
         # mask_in_backward=True applies the FInC gradient mask inside the weight-gradient kernel.  The reference clips
@@ -729,13 +686,16 @@ class FastFlowStep(_Chain):
             if unit.logdet_mode == "tensor":   # otherwise the unit reports 0.0 like the reference (fastflow.py:34-50)
                 ld = ld + unit.logdet(x)
             return y, ld
-        return self._fwd(self.fastflow_step, x)
+        return _forward_layers(self.fastflow_step, x)
+
+    def _reverse(self, x, want_logdet):
+        return _reverse_layers(self.fastflow_step, x, want_logdet)
 
     def reverse(self, x):
-        return self._rev(self.fastflow_step, x)
+        return self._reverse(x, False)[0]
 
     def reverse_and_logdet(self, x):
-        return _reverse_and_logdet(self.fastflow_step, x)
+        return self._reverse(x, True)
 
 
 class FastFlowLevel(nn.Module):
@@ -757,16 +717,17 @@ class FastFlowLevel(nn.Module):
             logdet = logdet + ld
         return x, z, logdet
 
+    def _reverse(self, x, z, want_logdet):
+        *layers, split = self.fastflow_level
+        x, ld = split._reverse(x, z, want_logdet)
+        x, ld_rest = _reverse_layers(layers, x, want_logdet)
+        return x, (ld + ld_rest if want_logdet else None)
+
     def reverse(self, x, z=None):
-        for layer in reversed(self.fastflow_level):
-            x = layer.reverse(x, z) if isinstance(layer, SplitPrior) else layer.reverse(x)
-        return x
+        return self._reverse(x, z, False)[0]
 
     def reverse_and_logdet(self, x, z=None):
-        split = self.fastflow_level[-1]
-        x, ld = split.reverse_and_logdet(x, z)
-        x, ld_rest = _reverse_and_logdet(self.fastflow_level[:-1], x)
-        return x, ld + ld_rest
+        return self._reverse(x, z, True)
 
 
 class FastFlow(nn.Module):
@@ -799,7 +760,7 @@ class FastFlow(nn.Module):
                 groups.setdefault(mod.n_channels, []).append(mod)
         for n_ch, convs in groups.items():
             Ws = torch.stack([c.W for c in convs])
-            lds = _SlogdetFn.apply(Ws) if n_ch <= 128 else torch.linalg.slogdet(Ws)[1]
+            lds = _SlogdetFn.apply(Ws) if _native_slogdet(Ws) else torch.linalg.slogdet(Ws)[1]
             for i, c in enumerate(convs):
                 c._ld_batched = lds[i]
 
@@ -824,29 +785,29 @@ class FastFlow(nn.Module):
         """x = the flow's inverse of the latents `zs` (sampled when None).  Differentiable in `zs` and every parameter
         the inverse uses (ops.finc_inverse says when a graph is recorded); `quantize=False` returns the continuous image before the final floor, which has zero gradient
         (Preprocess.reverse)."""
-        if zs is None:
-            zs = [self.base_distribution.sample(n_samples)[0]]
-        z = zs[-1]
-        for step in reversed(self.fastflow_step):
-            z = step.reverse(z)
-        x = self.squeeze.reverse(z)
-        for i, level in enumerate(reversed(self.fastflow_levels)):
-            x = level.reverse(x) if len(zs) == 1 else level.reverse(x, zs[-i - 2])
-        return self.preprocess.reverse(x, quantize=quantize)
+        return self._reverse(n_samples, zs, False, quantize)[0]
 
     def sample_with_log_prob(self, n_samples=1, zs=None):
         """(x, log_q[B]): x = reverse(n_samples, zs, quantize=False), the continuous image, and log_q its log-density
         under the model in nats, log N(every latent, the split-prior ones drawn inside included) - log|det dx/dz|.
         This is model.log_prob(x) with zero dequantisation noise, without a second pass.  Differentiable in `zs` and
         the parameters wherever reverse() records a graph (reverse-KL: E_q[log q(x) - log p*(x)])."""
+        return self._reverse(n_samples, zs, True)
+
+    def _reverse(self, n_samples, zs, want_logdet, quantize=False):
+        """(reverse(n_samples, zs, quantize=quantize), log_q or None unless `want_logdet`).  Latents not given are drawn
+        in this order: the base sample first, then the split priors from the last level to the first."""
         if zs is None:
             zs = [self.base_distribution.sample(n_samples)[0]]
-        z, logdet = _reverse_and_logdet(self.fastflow_step, zs[-1])
-        x = self.squeeze.reverse(z)
+        x, logdet = _reverse_layers(self.fastflow_step, zs[-1], want_logdet)
+        x = self.squeeze.reverse(x)
         for i, level in enumerate(reversed(self.fastflow_levels)):
-            x, ld = level.reverse_and_logdet(x) if len(zs) == 1 else level.reverse_and_logdet(x, zs[-i - 2])
-            logdet = logdet + ld
-        x, ld = self.preprocess.reverse_and_logdet(x)
+            x, ld = level._reverse(x, None if len(zs) == 1 else zs[-i - 2], want_logdet)
+            if want_logdet:
+                logdet = logdet + ld
+        x, ld = self.preprocess._reverse(x, want_logdet, quantize)
+        if not want_logdet:
+            return x, None
         return x, self.base_distribution.log_prob(zs[-1]) - (logdet + ld)
 
     def log_prob(self, x, bits_per_pixel=False):
