@@ -35,6 +35,49 @@ def test_library_exports_every_declared_symbol(lib_path):
     assert sorted(_native.SYMBOLS) == names
 
 
+def _header_prototypes():
+    """{name: (return type, [parameter types])} of every function prototype in the header, types as written"""
+    src = open(os.path.join(REPO, "include", "fincflow_b200.h")).read()
+    src = re.sub(r"/\*.*?\*/", "", src, flags=re.S)
+    protos = {}
+    for ret, name, params in re.findall(r"([A-Za-z_][\w \t]*?\**)\s*\b(finc_[a-z0-9_]+)\s*\(([^)]*)\)\s*;", src):
+        types = [re.sub(r"\s*\b\w+$", "", p.strip()) for p in params.split(",") if p.strip() not in ("", "void")]
+        protos[name] = (ret.strip(), types)
+    return protos
+
+
+def _ctype_of(decl, structs):
+    """the ctypes type a C type of the header binds to"""
+    from fincflow_b200 import _native
+
+    decl = " ".join(decl.replace("const", " ").replace("*", " * ").split())
+    if decl == "char *":
+        return ctypes.c_char_p
+    if decl.endswith("*"):
+        base = decl[:-1].strip()
+        return ctypes.POINTER(getattr(_native, base)) if base in structs else ctypes.c_void_p
+    return {"int": ctypes.c_int, "unsigned": ctypes.c_uint, "long": ctypes.c_long, "size_t": ctypes.c_size_t,
+            "float": ctypes.c_float}[decl]
+
+
+def test_signature_table_matches_the_header():
+    """return type and the number and C type of every parameter of every header function, against the binding's
+    one signature table"""
+    from fincflow_b200 import _native
+
+    src = open(os.path.join(REPO, "include", "fincflow_b200.h")).read()
+    structs = set(re.findall(r"typedef struct (\w+)", src))
+    protos = _header_prototypes()
+    assert sorted(protos) == _header_functions() == sorted(_native._SIGNATURES)
+    for name, (ret, params) in protos.items():
+        restype, argtypes = _native._SIGNATURES[name]
+        assert restype is _ctype_of(ret, structs), (name, ret, restype)
+        want = [_ctype_of(p, structs) for p in params]
+        assert len(argtypes) == len(want), (name, len(argtypes), len(want))
+        for k, (got, exp) in enumerate(zip(argtypes, want)):
+            assert got is exp, f"{name} parameter {k} ({params[k]}): {got} bound, {exp} declared"
+
+
 def test_abi_version_and_error_strings(lib_path):
     from fincflow_b200 import _native
 

@@ -1,6 +1,6 @@
 """FINC_DEBUG_TS=1 python tools/kernel_timeline.py -- per-CTA phase timestamps of the tiled kernels
 (debug aid; see finc_debug_timestamps in include/fincflow_b200.h)."""
-import ctypes, os, sys
+import os, sys
 os.environ["FINC_DEBUG_TS"] = "1"
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch
@@ -8,7 +8,6 @@ from fincflow_b200 import _native
 from fincflow_b200.fastflow import FastFlowUnit
 
 lib = _native.load()
-lib.finc_debug_timestamps.argtypes = [ctypes.c_void_p, ctypes.c_int]
 dev = torch.device("cuda:0")
 B = int(sys.argv[1]) if len(sys.argv) > 1 else 256
 NAMES = {"forward": ["entry", "weights staged", "first chunk landed", "chunk computed"],
